@@ -27,6 +27,7 @@ import time
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True      # the benchmark writes nothing into the tree it runs from (it may be read-only)
 
 import numpy as np  # noqa: E402
 
@@ -148,6 +149,30 @@ def same_pt(a, b):
     return a is not None and b is not None and int(a[1]) == int(b[1]) and np.array_equal(np.asarray(a[0], np.uint64), np.asarray(b[0], np.uint64))
 
 
+def words_f64(limbs):
+    """uint64 limbs (field elements, point coordinates in the library's Montgomery image) -> their 32-bit words, low word
+    first, as float64: exact, since every word is below 2^53"""
+    return np.ascontiguousarray(limbs, dtype=np.uint64).view(np.uint32).astype(np.float64)
+
+
+def point_f64(p):
+    """(xy, inf) as the library returns it -> the 16 words of x || y followed by the infinity flag"""
+    return np.append(words_f64(p[0]).reshape(16), float(p[1]))
+
+
+def proof_f64(name, l_vec, r_vec, final_key, c):
+    """an IpaPC::open proof: l_vec and r_vec (one point per round), final_comm_key (affine x || y) and c"""
+    return {f"{name}_l": np.stack([point_f64(p) for p in l_vec]), f"{name}_r": np.stack([point_f64(p) for p in r_vec]),
+            f"{name}_final_key": words_f64(final_key), f"{name}_c": words_f64(c)}
+
+
+def dump_outputs(outdir, outputs):
+    """--dump-outputs: one DIR/<name>.npy per result of the timed path, for comparing two builds output for output"""
+    os.makedirs(outdir, exist_ok=True)
+    for name, a in outputs.items():
+        np.save(os.path.join(outdir, f"{name}.npy"), np.asarray(a, dtype=np.float64))
+
+
 def run_reference(args, rank, world):
     """--impl reference: the ark-ec VariableBaseMSM restatement on host cores, same config / metric / unit."""
     if rank != 0:
@@ -173,8 +198,10 @@ def run_reference(args, rank, world):
         cref.msm_ark(0, pts, sc)
     t0 = time.perf_counter()
     for _ in range(args.steps):
-        cref.msm_ark(0, pts, sc)
+        res = cref.msm_ark(0, pts, sc)
     dt = (time.perf_counter() - t0) / args.steps
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, {"msm": point_f64(res)})
     mpts = n / dt / 1e6
     cores = ark_threads(n, cref.num_threads())
     print(json.dumps({
@@ -205,7 +232,11 @@ def main():
     ap.add_argument("--no-open", action="store_true", help="skip the IpaPC::open timing")
     ap.add_argument("--no-precompute", action="store_true", help="skip the per-key window table (one-shot bases)")
     ap.add_argument("--window-bits", type=int, default=0)
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write what the timed path computed in its last step as DIR/<name>.npy "
+                                                          "(float64: 32-bit words of the limbs; points end with their infinity flag)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     rank = int(os.environ.get("RANK", "0"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
@@ -285,7 +316,7 @@ def main():
     for a, b in evs:
         flush.zero_()
         a.record(stream)
-        step_dev()
+        res = step_dev()
         b.record(stream)
         if world == 1:
             for k, v in ctx.last_timings().items():
@@ -313,6 +344,7 @@ def main():
         dist.all_reduce(lt, op=dist.ReduceOp.SUM)
     t_dev_ms, t_e2e_ms = float(tt[0]), float(tt[1])
     launches = int(lt[0])
+    outputs = {"msm": point_f64(res), "msm_e2e": point_f64(res_e2e)} if rank == 0 else {}
 
     checks = {}
     # ---- parity of the timed multi-GPU step: every rank restates the MSM of its own shard on the CPU (oracle), the N affine
@@ -344,10 +376,11 @@ def main():
             for _ in range(5):
                 flush.zero_(); torch.cuda.synchronize()
                 t0 = time.perf_counter()
-                ok, _, _ = ctx.ipa_check_final_key(ipa_keys[k], ch, fk[0], fk[1])
+                ok, dxy, dinf = ctx.ipa_check_final_key(ipa_keys[k], ch, fk[0], fk[1])
                 ts.append((time.perf_counter() - t0) * 1e3)
                 assert ok
             decide[f"ipa_decide_tail_ms_2^{k}"] = round(statistics.median(ts), 4)
+            outputs[f"ipa_decide_tail_2^{k}"] = np.append(point_f64((dxy, dinf)), float(ok))     # final key, then accept
             if k == 18 and not args.no_cpu_baseline:
                 # CPU restatement of the same tail (compute_coeffs serial like upstream + VariableBaseMSM over windows), same key
                 from oracle import cref
@@ -394,6 +427,8 @@ def main():
         tdec = torch.tensor([statistics.median(ts)], dtype=torch.float64, device=dev)
         dist.all_reduce(tdec, op=dist.ReduceOp.MAX)
         decide[f"ipa_decide_tail_sharded_ms_2^{kk}"] = round(float(tdec[0]), 4)
+        if rank == 0:
+            outputs[f"ipa_final_key_sharded_2^{kk}"] = point_f64(fk)
         # config 5 strong scaling: ONE 2^20-point MSM sharded over all ranks (scalars resident in HBM)
         d_sl = d_sc[:s_cnt]
         for _ in range(3):
@@ -407,12 +442,14 @@ def main():
             flush.zero_()
             barrier()
             t0 = time.perf_counter()
-            dsh.msm_dev(d_sl, montgomery=False)
+            strong_res = dsh.msm_dev(d_sl, montgomery=False)
             barrier()
             ts.append((time.perf_counter() - t0) * 1e3)
         tdec = torch.tensor([statistics.median(ts)], dtype=torch.float64, device=dev)
         dist.all_reduce(tdec, op=dist.ReduceOp.MAX)
         decide[f"msm_sharded_strong_ms_2^{kk}"] = round(float(tdec[0]), 4)
+        if rank == 0:
+            outputs[f"msm_sharded_strong_2^{kk}"] = point_f64(strong_res)
         dkey.release()
         # ipa-pc-as prove hot path sharded: IpaPC::open at degree 2^20 with key / coefficients / z-vector sharded
         # cyclically (ShardedIpaOpen): per round one all-gather of 2 x 128-byte shares, last log2(N) rounds replicated
@@ -443,12 +480,14 @@ def main():
             for _ in range(3):
                 barrier()
                 t0 = time.perf_counter()
-                so.open(cf, z, squeeze_s, xi0_mont=xi0)
+                proof = so.open(cf, z, squeeze_s, xi0_mont=xi0)
                 barrier()
                 ts.append((time.perf_counter() - t0) * 1e3)
             tdec = torch.tensor([min(ts[1:])], dtype=torch.float64, device=dev)
             dist.all_reduce(tdec, op=dist.ReduceOp.MAX)
             decide[f"ipa_open_sharded_ms_2^{kk}"] = round(float(tdec[0]), 3)
+            if rank == 0:
+                outputs.update(proof_f64(f"ipa_open_sharded_2^{kk}", *proof[:4]))
             okey.release()
 
     # ---- ipa-pc-as prove hot path: IpaPC::open on device (metric string: prove ms at degree 2^18), one GPU
@@ -478,6 +517,7 @@ def main():
             ok, _, _ = ctx.ipa_check_final_key(ipa_keys[k], np.array(chs), fk, 0)     # the proof's final key passes the decider
             assert ok
             decide[f"ipa_open_ms_2^{k}"] = round(min(ts), 3)
+            outputs.update(proof_f64(f"ipa_open_2^{k}", l_vec, r_vec, fk, c))
 
         # ---- AS-shaped prove (examples/scaling-as.rs:91-103: 1 input + 2 copies of an accumulator, zk; src/ipa_pc_as/mod.rs:625-668):
         #      m = 3 succinct-check group equations (2k + 3 term one-shot MSMs), the combined check polynomial built, evaluated and
@@ -499,18 +539,22 @@ def main():
             for _ in range(2):
                 torch.cuda.synchronize()
                 t0 = time.perf_counter()
-                ctx.msm_oneshot_batch(ab.PALLAS, sc_pts_m, sc_scal_m, montgomery=False)   # succinct_check of every input / accumulator, one batched call
+                sc_res = ctx.msm_oneshot_batch(ab.PALLAS, sc_pts_m, sc_scal_m, montgomery=False)   # succinct_check of every input / accumulator, one batched call
                 sess, ev = ctx.ipa_open_begin_combined(ipa_keys[k], chm, al, zz, None, rp)
                 ctx.ipa_open_use_hiding_generator(sess, n, xi0)
-                xi, lr, nround = None, ctx.ipa_open_round(sess), 0
+                xi, lr, nround, l_vec, r_vec = None, ctx.ipa_open_round(sess), 0, [], []
                 while lr is not None:
                     xi = squeeze(xi, lr[0], lr[1])
+                    l_vec.append(lr[0]); r_vec.append(lr[1])
                     lr = ctx.ipa_open_fold_round(sess, xi)
                     nround += 1
                 fk, c = ctx.ipa_open_finish(sess)
                 ts.append((time.perf_counter() - t0) * 1e3)
             assert nround == k
             decide[f"ipa_as_prove_ms_2^{k}"] = round(min(ts), 3)
+            outputs.update(proof_f64(f"ipa_as_prove_2^{k}", l_vec, r_vec, fk, c))
+            outputs[f"ipa_as_prove_2^{k}_succinct_msms"] = np.stack([point_f64(p) for p in zip(*sc_res)])
+            outputs[f"ipa_as_prove_2^{k}_evaluation"] = words_f64(ev)
             decide["ipa_as_prove_shape"] = f"m = {m_as} (1 input + 2 accumulator copies), zk, degree 2^{k}: {m_as} succinct-check equations + combine + evaluate + open"
 
         # ---- CPU restatement of the opening / the AS-shaped prove on a BOUNDED sample (degree 2^12: the CPU folds the key
@@ -624,6 +668,8 @@ def main():
     out.update(decide)
     if extras_cpu:
         out["cpu_baselines_protocol"] = extras_cpu
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, outputs)
     print(json.dumps(out), flush=True)
     if world > 1:
         dist.barrier()

@@ -25,11 +25,9 @@ def build_harness():
 
 
 def test_harness_builds_and_refuses_without_gpu():
-    import torch
+    """the harness runs with every CUDA device hidden, so the refusal is observable on a machine with a GPU too"""
     exe = build_harness()
-    if torch.cuda.is_available():
-        pytest.skip("a GPU is present")
-    p = subprocess.run([exe], capture_output=True, text=True, timeout=120)
+    p = subprocess.run([exe], capture_output=True, text=True, timeout=120, env=dict(os.environ, CUDA_VISIBLE_DEVICES=""))
     assert p.returncode == 3 and "NO_GPU" in p.stdout
 
 
