@@ -72,8 +72,9 @@ struct accmsm_ctx {
     std::vector<GroupWorker *> workers;
     std::unordered_map<uint64_t, GroupKey *> gkeys;
     std::unordered_map<uint64_t, GroupCsr *> gcsrs;
-    std::unordered_map<uint64_t, uint64_t> gsessions;   // IpaPC::open sessions run on child 0: group id -> child session id
+    std::unordered_map<uint64_t, struct GroupIpaSession *> gsessions;   // IpaPC::open sessions sharded across the children
     std::vector<char> peer_ok;                           // child g can store straight into child 0's memory
+    std::vector<char> peer_read;                         // [i * children + j]: child i's kernels can read child j's memory
     void *d_gather = nullptr;                            // on child 0's device: partial sums of all children, rank-major
     size_t min_shard = size_t(1) << 16;                  // keys are cut into shards of at least this many points
     int device = 0;
@@ -976,6 +977,17 @@ int group_csr_matvec_commit(accmsm_ctx *g, uint64_t key_handle, uint64_t csr_han
                             const uint64_t *witness, size_t n_witness, size_t hiding_index, const uint64_t *blinders_mont,
                             uint64_t *const *out_vecs, uint64_t *out_xy, uint8_t *out_inf);
 int group_open_key(accmsm_ctx *g, uint64_t handle, uint64_t *kid0_handle);     // full key on child 0 for IpaPC::open sessions
+// IpaPC::open sessions sharded cyclically across the children of a group (multi_api.inc).  GROUP_IPA_UNSHARDED: the
+// opening is too small to shard / the id is not a sharded session, and child 0 serves the call as before.
+constexpr int GROUP_IPA_UNSHARDED = 1;
+int group_ipa_begin(accmsm_ctx *g, uint64_t handle, const uint64_t *coeffs_mont, size_t n_coeffs, int k, const uint64_t point_mont[4],
+                    const uint64_t h_prime_xy[8], const uint64_t *challenges_mont, int m, const uint64_t *alphas_mont,
+                    const uint64_t *random_poly_mont, size_t n_random, uint64_t *session, uint64_t *eval_out);
+int group_ipa_use_hiding_generator(accmsm_ctx *g, uint64_t session, size_t h_index, const uint64_t xi0_mont[4]);
+int group_ipa_round(accmsm_ctx *g, uint64_t session, const uint64_t *xi_mont, uint64_t l_xy[8], uint8_t *l_inf, uint64_t r_xy[8],
+                    uint8_t *r_inf, int *done);
+int group_ipa_fold(accmsm_ctx *g, uint64_t session, const uint64_t xi_mont[4], const uint64_t xi_inv_mont[4]);
+int group_ipa_finish(accmsm_ctx *g, uint64_t session, uint64_t final_key_xy[8], uint64_t c_mont[4]);
 inline bool is_group(const accmsm_ctx *ctx) { return ctx && !ctx->kids.empty(); }
 #define GROUP_NO_DEV(ctx, name) do { if (is_group(ctx)) return fail_arg(ctx, name ": device-pointer entry points need a single-device ctx (accmsm_device_ctx)"); } while (0)
 

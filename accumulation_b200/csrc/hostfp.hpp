@@ -70,6 +70,20 @@ inline void mul(const Modulus &M, const uint64_t a[4], const uint64_t b[4], uint
     for (int j = 0; j < 4; j++) r[j] = ge ? d[j] : t[j];
 }
 
+// r = a + b mod m; inputs < m, output < m (m < 2^255: the sum does not carry out of 256 bits).  r may alias a or b.
+inline void add(const Modulus &M, const uint64_t a[4], const uint64_t b[4], uint64_t r[4]) {
+    uint64_t s[4], d[4];
+    u128 c = 0;
+    for (int j = 0; j < 4; j++) { c += (u128)a[j] + b[j]; s[j] = (uint64_t)c; c >>= 64; }
+    u128 br = 0;
+    for (int j = 0; j < 4; j++) {
+        u128 x = (u128)s[j] - M.m[j] - (uint64_t)br;
+        d[j] = (uint64_t)x;
+        br = (x >> 64) & 1;
+    }
+    for (int j = 0; j < 4; j++) r[j] = br ? s[j] : d[j];
+}
+
 // a^(m - 2) in the Montgomery domain: maps the image a R to a^-1 R; inv(0) = 0.  4-bit fixed windows: 252 squarings + ~70 products.
 inline void inv(const Modulus &M, const uint64_t a[4], uint64_t r[4]) {
     uint64_t e[4] = {M.m[0] - 2, M.m[1], M.m[2], M.m[3]};     // m[0] ends in ...01: no borrow

@@ -271,4 +271,29 @@ __global__ void __launch_bounds__(FOLD_THREADS) k_fold_combine(const xyzz_t *__r
     store_fe(&out[p].x, a.x); store_fe(&out[p].y, a.y);
 }
 
+// Cyclic key layout of one shard of a multi-GPU opening: out[t] = key[offset + (t << log_stride)], read from the
+// contiguous point ranges [start[s], start[s] + count[s]) that hold the key (peer pointers over NVLink, or a local copy
+// of one range).  Indices that fall in none of the given ranges are left untouched, so one launch per copied range
+// fills the layout piece by piece.
+constexpr int CYCLIC_MAX_SRC = 16;
+struct CyclicSrc {
+    const affine_t *xy[CYCLIC_MAX_SRC];
+    uint64_t start[CYCLIC_MAX_SRC], count[CYCLIC_MAX_SRC];
+    int n_src;
+};
+__global__ void __launch_bounds__(256) k_cyclic_gather(CyclicSrc src, uint64_t offset, uint32_t log_stride, uint64_t n_out,
+                                                        affine_t *__restrict__ out) {
+    const uint64_t t = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (t >= n_out) return;
+    const uint64_t i = offset + (t << log_stride);
+    for (int s = 0; s < src.n_src; s++) {
+        if (i < src.start[s] || i - src.start[s] >= src.count[s]) continue;
+        const uint4 *p = reinterpret_cast<const uint4 *>(src.xy[s] + (i - src.start[s]));
+        uint4 *o = reinterpret_cast<uint4 *>(out + t);
+        const uint4 a = p[0], b = p[1], c = p[2], d = p[3];
+        o[0] = a; o[1] = b; o[2] = c; o[3] = d;
+        return;
+    }
+}
+
 }  // namespace accmsm

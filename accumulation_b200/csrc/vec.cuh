@@ -19,20 +19,28 @@ struct VecPtrs {
 // of the challenges selected by the low L / high k - L index bits.  One product per coefficient instead of ~k/2
 // (the element-wise kernel is then bound by its 32-byte store, not by the multiplier); the tables (<= 2 x 2^11 entries
 // per polynomial) stay in L1/L2.  alphas (nullable) are folded into the hi tables: hi_i *= alpha_i.
+// Cyclic shard form (log_shards > 0): the tables cover only coefficients shard_index + 2^log_shards t, t < 2^(k -
+// log_shards), indexed by t.  The low log_shards index bits are then fixed, so the product of their challenges is one
+// constant per polynomial, folded into the hi tables like alpha.  (0, 0) is the whole polynomial.
 template <int FIELD>
 __global__ void __launch_bounds__(256) k_coeff_tables(const uint8_t *__restrict__ challenges, int m, int k, int L,
                                                        const uint8_t *__restrict__ alphas, uint8_t *__restrict__ lo,
-                                                       uint8_t *__restrict__ hi) {
+                                                       uint8_t *__restrict__ hi, uint32_t log_shards, uint32_t shard_index) {
     using F = Fp<FIELD>;
-    const uint32_t n_lo = 1u << L, n_hi = 1u << (k - L), per = n_lo + n_hi;
+    const int kl = k - (int)log_shards;
+    const uint32_t n_lo = 1u << L, n_hi = 1u << (kl - L), per = n_lo + n_hi;
     uint32_t t = blockIdx.x * blockDim.x + threadIdx.x;
     if (t >= per * (uint32_t)m) return;
     const uint32_t i = t / per, e = t % per;
     const uint8_t *ch = challenges + (size_t)i * k * 32;
     const bool is_lo = e < n_lo;
     const uint32_t idx = is_lo ? e : e - n_lo;
-    const int b0 = is_lo ? 0 : L, nb = is_lo ? L : k - L;
+    const int b0 = (int)log_shards + (is_lo ? 0 : L), nb = is_lo ? L : kl - L;
     fe_t acc = (!is_lo && alphas) ? load_fe(alphas + (size_t)i * 32) : F::one();
+    if (!is_lo) {
+        for (uint32_t b = 0; b < log_shards; b++)
+            if ((shard_index >> b) & 1u) acc = F::mul(acc, load_fe(ch + (size_t)(k - 1 - (int)b) * 32));
+    }
     for (int b = 0; b < nb; b++) {             // index bit b0 + b  <->  challenge k - 1 - (b0 + b)
         if ((idx >> b) & 1u) acc = F::mul(acc, load_fe(ch + (size_t)(k - 1 - (b0 + b)) * 32));
     }

@@ -54,8 +54,13 @@ int  accmsm_init(accmsm_ctx **out, int device);
  * on its range and stores one un-normalised 128-byte partial per result into device 0's memory over NVLink (peer store from
  * the last kernel; cudaMemcpyPeer without peer access); device 0 adds them and normalises.  accmsm_ipa_final_key expands
  * h(X) per range with no exchange; accmsm_hp_decide / accmsm_hp_product_poly_comm / accmsm_csr_matvec_commit and the
- * element-wise accmsm_vec_* calls shard by the same index ranges (CSR rows with z replicated).  IpaPC::open sessions run on
- * device 0 over a copy of the whole key assembled by peer copies.  The device-pointer (`*_dev`) entry points need a
+ * element-wise accmsm_vec_* calls shard by the same index ranges (CSR rows with z replicated).  The accmsm_ipa_open_* calls
+ * (begin, begin_combined and begin_shard with log_shards == 0 and no z_scale) shard an opening of 2^k coefficients
+ * cyclically over G devices, G the largest power of two <= n_dev and <= 2^k with 2^k / G >= min_shard: device g holds
+ * key[g::G] and coeffs[g::G] for the first k - log2 G rounds (one 2 x 128-byte exchange per device per round, combined on
+ * device 0), device 0 runs the last log2 G rounds; the proof and eval_out are bit-identical to a single-device session.
+ * Smaller openings, and begin_shard with log_shards > 0, run on device 0 over a copy of the whole key assembled by peer
+ * copies.  The device-pointer (`*_dev`) entry points need a
  * single-device ctx: accmsm_device_ctx(group, i).  This is what the single-process Rust callers
  * (src/ipa_pc_as/mod.rs:836-845, src/hp_as/mod.rs:910-918, src/r1cs_nark_as/mod.rs:1052-1097) bind. */
 int  accmsm_init_multi(accmsm_ctx **out, const int *devices, int n_dev);

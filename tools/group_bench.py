@@ -3,16 +3,21 @@ keys sharded inside the library (no torch.distributed, no NCCL).  One JSON line 
   weak   : one G * 2^20-point MSM from pinned host scalars (the bench.py e2e shape), Mpts/s
   strong : one 2^20-point MSM, the ipa-pc-as decide tail at degree 2^20 / 2^18 (config 4), hp-as decide with 2^16-element
            vectors (config 2), r1cs-nark A z / B z / C z + three commitments at 2^16 constraints (config 3), ms
+  open   : IpaPC::open (h' by index, fold_round per round) at 2^20 and 2^18, sharded across the group at the default
+           min_shard on >= 2 GPUs, and at 2^14, which stays on child 0: a workload on each side of the rule, ms
 Every result is compared with the single-device ctx (which the GPU suite pins to the oracle) before it is printed.
-Usage: python tools/group_bench.py [--gpus 1,2,4,8]"""
+Usage: python tools/group_bench.py [--gpus 1,2,4,8] [--devices 0,0]   (--devices: one group over exactly these devices;
+a device listed twice makes a virtual group on one GPU, which runs every path but measures no multi-GPU speed)"""
 import argparse, json, os, statistics, sys, time
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 import numpy as np
 import accumulation_b200 as ab
 from tests.test_gpu_fused import scaling_nark_matrices
+from tests.test_gpu_ipa_open import sponge_stand_in
 
 ap = argparse.ArgumentParser()
 ap.add_argument("--gpus", default="1,2,4,8")
+ap.add_argument("--devices", default=None)
 ap.add_argument("--reps", type=int, default=10)
 args = ap.parse_args()
 SEED = 0xACC5
@@ -46,6 +51,23 @@ ref_msm = ref.msm(key1, sc20, montgomery=False)
 ch20 = rand_scalars(20, SEED + 77)
 ref_fk20 = ref.ipa_final_key(key1, ch20)
 ref_fk18 = ref.ipa_final_key(key1, ch20[:18])
+OPEN_LOGS = (20, 18, 14)
+open_coeffs = rand_scalars(N20, SEED + 31)
+open_z, open_xi0 = rand_scalars(1, SEED + 32).reshape(4), rand_scalars(1, SEED + 33).reshape(4)
+open_squeeze = sponge_stand_in(1)       # curve 0: scalars in field 1
+
+
+def open_proof(c, B, lk):
+    ck = ab.CommitterKey(B, N20)        # the hiding generator is base N20
+    return ab.InnerProductArgPC.open(ck, open_coeffs[:1 << lk], open_z, None, open_squeeze, log_d=lk, xi0=open_xi0)
+
+
+def same_proof(a, b):
+    return (all(same(x, y) for x, y in zip(a[0] + a[1], b[0] + b[1])) and len(a[0]) == len(b[0])
+            and np.array_equal(a[2], b[2]) and np.array_equal(a[3], b[3]))
+
+
+ref_open = {lk: open_proof(ref, key1, lk) for lk in OPEN_LOGS}
 L = 1 << 16
 keyL = ref.register_synthetic_bases(0, SEED + 9, L + 1); keyL.precompute()
 a, b = rand_scalars(L, 11), rand_scalars(L, 12)
@@ -56,9 +78,11 @@ inp, wit, bl = rand_scalars(n_in, 21), rand_scalars(n_wit, 22), rand_scalars(3, 
 csr1 = ref.register_csr(1, mats)
 ref_vecs, ref_cxy, ref_cinf = ref.csr_matvec_commit(keyL, csr1, 3, L, inp, wit, hiding_index=L, blinders=bl)
 
-for G in [int(g) for g in args.gpus.split(",")]:
-    g = ab.Context(devices=list(range(G))) if G > 1 else ab.Context(0)
-    rec = {"gpus": G, "process": "one process, accmsm_init_multi" if G > 1 else "one process, accmsm_init"}
+groups = [[int(d) for d in args.devices.split(",")]] if args.devices else [list(range(int(G))) for G in args.gpus.split(",")]
+for devs in groups:
+    G = len(devs)
+    g = ab.Context(devices=devs) if G > 1 else ab.Context(devs[0])
+    rec = {"gpus": G, "devices": devs, "process": "one process, accmsm_init_multi" if G > 1 else "one process, accmsm_init"}
     # ---- weak: one G * 2^20-point MSM, host scalars (pinned), whole call timed
     n = N20 * G
     kw = g.register_synthetic_bases(0, SEED, n); kw.precompute()
@@ -83,6 +107,9 @@ for G in [int(g) for g in args.gpus.split(",")]:
     rec.update({"decide_tail_2^18_ms": round(t, 4), "decide_18_verified": same(res, ref_fk18)})
     bad = ch20.copy(); bad[7, 1] ^= np.uint64(8)
     rec["decide_rejects_corrupted"] = not g.ipa_check_final_key(ks, bad, ref_fk20[0], ref_fk20[1])[0]
+    for lk in OPEN_LOGS:
+        t, res = timed(lambda: open_proof(g, ks, lk), args.reps)
+        rec.update({f"ipa_open_2^{lk}_ms": round(t, 4), f"ipa_open_{lk}_verified": same_proof(res, ref_open[lk])})
     ks.release()
     # ---- config 2 / 3 at 2^16 (below the default shard size: min_shard lowered so the group really splits them)
     g.set_min_shard(1 << 13) if G > 1 else None
