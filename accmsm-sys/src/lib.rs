@@ -266,6 +266,31 @@ impl<'k> IpaOpenSession<'k> {
         key.ctx.check(unsafe { ffi::accmsm_ipa_open_use_hiding_generator(key.ctx.raw, id, h, (xi0.0).0.as_ptr()) })?;
         Ok(IpaOpenSession { key, id, finished: false })
     }
+    /// zk opening (`MakeZK::Enabled`): begin without xi_0, which upstream squeezes from `C'` only after the hiding step:
+    /// `begin_zk` -> `hide` -> hiding_comm; alpha = sponge(C, z, v, hiding_comm); `hiding_challenge(alpha)`;
+    /// `C' = C + alpha hiding_comm - (r + alpha rho) s` and xi_0 on the host; `use_hiding_generator(xi_0)`; then the rounds.
+    pub fn begin_zk<S: Fp256Parameters>(key: &'k GpuKey, coeffs: &[Fp256<S>], log_d: usize, point: Fp256<S>) -> Result<Self> {
+        let mut id = 0u64;
+        key.ctx.check(unsafe { ffi::accmsm_ipa_open_begin(key.ctx.raw, key.handle, limbs_of(coeffs), coeffs.len(), log_d as c_int, (point.0).0.as_ptr(), std::ptr::null(), &mut id) })?;
+        Ok(IpaOpenSession { key, id, finished: false })
+    }
+    /// The random polynomial (<= 2^log_d coefficients) is shifted on the device to vanish at the point and committed:
+    /// returns `hiding_comm = cm_commit(comm_key, hiding', Some(s), Some(rho))` with s the key's base `s_index`.
+    pub fn hide<P: GpuCurve + GpuBase, S: Fp256Parameters>(&mut self, hiding: &[Fp256<S>], s_index: usize, rho: Fp256<S>) -> Result<GroupAffine<P>> {
+        let (mut xy, mut inf) = ([0u64; 8], 0u8);
+        self.key.ctx.check(unsafe {
+            ffi::accmsm_ipa_open_hide(self.key.ctx.raw, self.id, limbs_of(hiding), hiding.len(), s_index, (rho.0).0.as_ptr(), xy.as_mut_ptr(), &mut inf)
+        })?;
+        Ok(affine_from::<P>(&xy, inf))
+    }
+    /// `P += alpha * hiding'` on the device (enqueued only).
+    pub fn hiding_challenge<S: Fp256Parameters>(&mut self, alpha: Fp256<S>) -> Result<()> {
+        self.key.ctx.check(unsafe { ffi::accmsm_ipa_open_hiding_challenge(self.key.ctx.raw, self.id, (alpha.0).0.as_ptr()) })
+    }
+    /// `h' = xi_0 * h` with h the key's base `h_index`; before the first round.
+    pub fn use_hiding_generator<S: Fp256Parameters>(&mut self, h_index: usize, xi0: Fp256<S>) -> Result<()> {
+        self.key.ctx.check(unsafe { ffi::accmsm_ipa_open_use_hiding_generator(self.key.ctx.raw, self.id, h_index, (xi0.0).0.as_ptr()) })
+    }
     pub fn round<P: GpuCurve + GpuBase>(&mut self) -> Result<(GroupAffine<P>, GroupAffine<P>)> {
         let (mut l, mut r, mut li, mut ri) = ([0u64; 8], [0u64; 8], 0u8, 0u8);
         self.key.ctx.check(unsafe { ffi::accmsm_ipa_open_round(self.key.ctx.raw, self.id, l.as_mut_ptr(), &mut li, r.as_mut_ptr(), &mut ri) })?;

@@ -354,6 +354,22 @@ class Context:
                     "ipa_open_begin_combined")
         return int(sess.value), ev
 
+    def ipa_open_hide(self, session: int, hiding_coeffs_mont, s_index: int, hiding_rand_mont):
+        """zk opening, before the first round: the random polynomial (shifted on the device to vanish at the point) and its
+        commitment cm_commit(key, hiding') + rho * key[s_index] -> (hiding_comm_xy, inf)"""
+        hc = _u64(hiding_coeffs_mont).reshape(-1, 4)
+        out = np.empty(8, dtype=np.uint64)
+        inf = C.c_uint8(0)
+        self._check(self._lib.accmsm_ipa_open_hide(self._h, C.c_uint64(session), _p(hc) if hc.shape[0] else None, C.c_size_t(hc.shape[0]),
+                                                   C.c_size_t(s_index), _p(_u64(hiding_rand_mont)), _p(out), C.byref(inf)),
+                    "ipa_open_hide")
+        return out, int(inf.value)
+
+    def ipa_open_hiding_challenge(self, session: int, alpha_mont):
+        """zk opening: coeffs += alpha * hiding' on the device (after ipa_open_hide, before the first round)"""
+        self._check(self._lib.accmsm_ipa_open_hiding_challenge(self._h, C.c_uint64(session), _p(_u64(alpha_mont))),
+                    "ipa_open_hiding_challenge")
+
     def ipa_open_round(self, session: int):
         l, r = np.empty(8, dtype=np.uint64), np.empty(8, dtype=np.uint64)
         li, ri = C.c_uint8(0), C.c_uint8(0)
@@ -543,8 +559,8 @@ class Bases:
 
 
 from .mirror import (  # noqa: E402
-    ASForHadamardProducts, CommitterKey, InnerProductArgPC, PedersenCommitment, R1CSNark, SuccinctCheckPolynomial, matrix_vec_mul,
+    ASForHadamardProducts, CommitterKey, InnerProductArgPC, PedersenCommitment, R1CSNark, SuccinctCheckPolynomial, ZkHiding, matrix_vec_mul,
 )
 
 __all__ = ["Context", "Bases", "pinned_array", "release_pinned", "AccmsmError", "PALLAS", "VESTA", "FP", "FQ", "scalar_field", "PedersenCommitment",
-           "CommitterKey", "InnerProductArgPC", "SuccinctCheckPolynomial", "ASForHadamardProducts", "R1CSNark", "matrix_vec_mul"]
+           "CommitterKey", "InnerProductArgPC", "SuccinctCheckPolynomial", "ZkHiding", "ASForHadamardProducts", "R1CSNark", "matrix_vec_mul"]

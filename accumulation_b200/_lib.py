@@ -15,7 +15,7 @@ SYMBOLS = [
     "accmsm_register_bases", "accmsm_release_bases", "accmsm_register_synthetic_bases", "accmsm_download_bases", "accmsm_precompute_bases", "accmsm_register_bases_compressed", "accmsm_serialize_bases",
     "accmsm_msm", "accmsm_msm_oneshot", "accmsm_msm_oneshot_batch", "accmsm_msm_batch", "accmsm_commit", "accmsm_msm_dev", "accmsm_msm_partial_dev", "accmsm_msm_partial", "accmsm_combine_partials_dev", "accmsm_combine_partials_batch_dev",
     "accmsm_ipa_final_key", "accmsm_ipa_check_final_key", "accmsm_ipa_final_key_partial_dev",
-    "accmsm_ipa_open_begin", "accmsm_ipa_open_begin_combined", "accmsm_ipa_open_use_hiding_generator", "accmsm_ipa_open_round", "accmsm_ipa_open_fold", "accmsm_ipa_open_fold_round", "accmsm_ipa_open_finish", "accmsm_ipa_open_begin_shard", "accmsm_ipa_open_round_partial_dev",
+    "accmsm_ipa_open_begin", "accmsm_ipa_open_begin_combined", "accmsm_ipa_open_use_hiding_generator", "accmsm_ipa_open_round", "accmsm_ipa_open_fold", "accmsm_ipa_open_fold_round", "accmsm_ipa_open_finish", "accmsm_ipa_open_begin_shard", "accmsm_ipa_open_round_partial_dev", "accmsm_ipa_open_hide", "accmsm_ipa_open_hiding_challenge",
     "accmsm_compute_coeffs", "accmsm_combine_check_polys", "accmsm_poly_evaluate",
     "accmsm_hp_decide", "accmsm_hp_decide_partial_dev", "accmsm_hp_product_poly_comm", "accmsm_hp_product_poly_comm_partial_dev", "accmsm_csr_matvec_commit_partial_dev", "accmsm_register_csr", "accmsm_release_csr", "accmsm_csr_matvec_commit",
     "accmsm_vec_hadamard", "accmsm_vec_scale", "accmsm_vec_lincomb", "accmsm_vec_tvecs", "accmsm_csr_matvec",

@@ -988,6 +988,9 @@ int group_ipa_round(accmsm_ctx *g, uint64_t session, const uint64_t *xi_mont, ui
                     uint8_t *r_inf, int *done);
 int group_ipa_fold(accmsm_ctx *g, uint64_t session, const uint64_t xi_mont[4], const uint64_t xi_inv_mont[4]);
 int group_ipa_finish(accmsm_ctx *g, uint64_t session, uint64_t final_key_xy[8], uint64_t c_mont[4]);
+int group_ipa_hide(accmsm_ctx *g, uint64_t session, const uint64_t *hiding_mont, size_t n_hiding, size_t s_index,
+                   const uint64_t rho_mont[4], uint64_t comm_xy[8], uint8_t *comm_inf);
+int group_ipa_hiding_challenge(accmsm_ctx *g, uint64_t session, const uint64_t alpha_mont[4]);
 inline bool is_group(const accmsm_ctx *ctx) { return ctx && !ctx->kids.empty(); }
 #define GROUP_NO_DEV(ctx, name) do { if (is_group(ctx)) return fail_arg(ctx, name ": device-pointer entry points need a single-device ctx (accmsm_device_ctx)"); } while (0)
 

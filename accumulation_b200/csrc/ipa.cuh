@@ -128,6 +128,23 @@ __global__ void __launch_bounds__(256) k_ipa_fold_scalars(uint8_t *__restrict__ 
     store_fe(z0, F::add(load_fe(z0), F::mul(x, load_fe(z + (size_t)(i + h) * 32))));
 }
 
+// zk opening: hiding[0] -= e, so that the hiding polynomial vanishes at the point (one thread)
+template <int FIELD>
+__global__ void k_ipa_hide_adjust(uint8_t *__restrict__ hiding, const uint8_t *__restrict__ e) {
+    store_fe(hiding, Fp<FIELD>::sub(load_fe(hiding), load_fe(e)));
+}
+// zk opening: coeffs[i] += alpha * hiding[i] once alpha is squeezed from (C, z, v, hiding_comm); alpha travels as a kernel
+// argument like the round challenges
+template <int FIELD>
+__global__ void __launch_bounds__(256) k_ipa_hide_fold(uint8_t *__restrict__ coeffs, const uint8_t *__restrict__ hiding,
+                                                        uint32_t n, fe_t alpha) {
+    using F = Fp<FIELD>;
+    uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= n) return;
+    uint8_t *c = coeffs + (size_t)i * 32;
+    store_fe(c, F::add(load_fe(c), F::mul(alpha, load_fe(hiding + (size_t)i * 32))));
+}
+
 
 // ------------------------------------------------------------------------------------------------
 // Folded-key materialisation.  The unfolded rounds above cost one MSM over ALL n0 / 2 pairs per job in every round,

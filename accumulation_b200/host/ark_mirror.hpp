@@ -72,9 +72,12 @@ private:
 // the base after the last generator, so commit(elems, Some(r)) is one pass of the device MSM.
 class CommitterKey {
 public:
+    // s (ipa_pc::CommitterKey::s, needs the hiding generator h): registered after h, so a zk opening's hiding_comm is one pass
     CommitterKey(std::shared_ptr<Context> ctx, int curve, const std::vector<Affine> &generators,
-                 const std::optional<Affine> &hiding_generator = std::nullopt, bool precompute = true)
-        : ctx_(std::move(ctx)), curve_(curve), n_(generators.size()), has_hiding_(hiding_generator.has_value()) {
+                 const std::optional<Affine> &hiding_generator = std::nullopt, bool precompute = true,
+                 const std::optional<Affine> &s = std::nullopt)
+        : ctx_(std::move(ctx)), curve_(curve), n_(generators.size()), has_hiding_(hiding_generator.has_value()), has_s_(s.has_value()) {
+        if (s && !hiding_generator) throw AccmsmError("CommitterKey: s follows the hiding generator h; pass both");
         std::vector<uint64_t> xy;
         std::vector<uint8_t> inf;
         xy.reserve((n_ + 1) * 8);
@@ -85,6 +88,7 @@ public:
         };
         for (const auto &g : generators) push(g);
         if (hiding_generator) push(*hiding_generator);
+        if (s) push(*s);
         ctx_->check(accmsm_register_bases(ctx_->raw(), curve, xy.data(), inf.data(), inf.size(), &handle_), "register_bases");
         if (precompute) ctx_->check(accmsm_precompute_bases(ctx_->raw(), handle_, 0), "precompute_bases");
     }
@@ -96,12 +100,13 @@ public:
     uint64_t handle() const { return handle_; }
     size_t hiding_index() const { return n_; }
     bool has_hiding() const { return has_hiding_; }
+    std::optional<size_t> s_index() const { return has_s_ ? std::optional<size_t>(n_ + 1) : std::nullopt; }
     const std::shared_ptr<Context> &ctx() const { return ctx_; }
 private:
     std::shared_ptr<Context> ctx_;
     int curve_;
     size_t n_;
-    bool has_hiding_;
+    bool has_hiding_, has_s_;
     uint64_t handle_ = 0;
 };
 
@@ -156,6 +161,8 @@ struct IpaProofCore {             // the fields of ipa_pc::Proof produced by the
     Affine final_comm_key;
     Fe c{};
     std::vector<Fe> round_challenges;
+    std::optional<Affine> hiding_comm;   // zk opening: the proof's hiding_comm, and the alpha squeezed from it (rand = r + alpha rho
+    Fe hiding_alpha{};                   // and C' = C + alpha hiding_comm - rand s stay with the caller, as upstream)
 };
 
 struct InnerProductArgPC {
@@ -220,6 +227,44 @@ struct InnerProductArgPC {
         }
         uint64_t fk[8];
         ck.ctx()->check(accmsm_ipa_open_finish(ck.ctx()->raw(), sess, fk, p.c.data()), "ipa_open_finish");
+        p.final_comm_key = affine_from(fk, 0);
+        return p;
+    }
+    // zk form (MakeZK::Enabled): before the first round the random polynomial `hiding` (<= 2^log_d coefficients from the caller's
+    // rng) is shifted on the device to vanish at the point and committed with (s, rho); alpha_of(hiding_comm) is the host sponge
+    // over (C, z, v, hiding_comm); xi0_of(hiding_comm, alpha) returns xi_0, which the caller squeezes from C'.  h' = xi_0 * h.
+    static IpaProofCore open_zk(const CommitterKey &ck, const std::vector<Fe> &combined_coeffs, int log_d, const Fe &point,
+                                const std::vector<Fe> &hiding, const Fe &rho, const std::function<Fe(const Affine &)> &alpha_of,
+                                const std::function<Fe(const Affine &, const Fe &)> &xi0_of,
+                                const std::function<Fe(const Affine &, const Affine &)> &round_challenge) {
+        if (!ck.s_index()) throw AccmsmError("open_zk: the key has no s (CommitterKey(.., s))");
+        uint64_t sess = 0;
+        accmsm_ctx *c = ck.ctx()->raw();
+        ck.ctx()->check(accmsm_ipa_open_begin(c, ck.handle(), combined_coeffs.empty() ? nullptr : combined_coeffs[0].data(),
+                                              combined_coeffs.size(), log_d, point.data(), nullptr, &sess), "ipa_open_begin");
+        IpaProofCore p;
+        uint64_t fk[8], xy[8]; uint8_t inf = 0;
+        try {
+            ck.ctx()->check(accmsm_ipa_open_hide(c, sess, hiding.empty() ? nullptr : hiding[0].data(), hiding.size(), *ck.s_index(), rho.data(),
+                                                 xy, &inf), "ipa_open_hide");
+            p.hiding_comm = affine_from(xy, inf);
+            p.hiding_alpha = alpha_of(*p.hiding_comm);
+            ck.ctx()->check(accmsm_ipa_open_hiding_challenge(c, sess, p.hiding_alpha.data()), "ipa_open_hiding_challenge");
+            const Fe xi0 = xi0_of(*p.hiding_comm, p.hiding_alpha);
+            ck.ctx()->check(accmsm_ipa_open_use_hiding_generator(c, sess, ck.hiding_index(), xi0.data()), "ipa_open_use_hiding_generator");
+        } catch (...) {
+            accmsm_ipa_open_finish(c, sess, fk, p.c.data());      // releases the session
+            throw;
+        }
+        uint64_t l[8], rr[8]; uint8_t li = 0, ri = 0; int done = log_d == 0;
+        if (!done) ck.ctx()->check(accmsm_ipa_open_round(c, sess, l, &li, rr, &ri), "ipa_open_round");
+        while (!done) {
+            p.l_vec.push_back(affine_from(l, li)); p.r_vec.push_back(affine_from(rr, ri));
+            Fe xi = round_challenge(p.l_vec.back(), p.r_vec.back());
+            p.round_challenges.push_back(xi);
+            ck.ctx()->check(accmsm_ipa_open_fold_round(c, sess, xi.data(), l, &li, rr, &ri, &done), "ipa_open_fold_round");
+        }
+        ck.ctx()->check(accmsm_ipa_open_finish(c, sess, fk, p.c.data()), "ipa_open_finish");
         p.final_comm_key = affine_from(fk, 0);
         return p;
     }

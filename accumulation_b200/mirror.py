@@ -7,7 +7,7 @@ this file, used by the Rust-side integration, is `accumulation_b200/host/ark_mir
 from __future__ import annotations
 
 from dataclasses import dataclass
-from typing import List, Optional, Sequence
+from typing import Callable, List, Optional, Sequence
 
 import numpy as np
 
@@ -17,20 +17,24 @@ class CommitterKey:
     """trivial_pc::CommitterKey{generators, hiding_generator} / ipa_pc::CommitterKey{comm_key, h, s}.
 
     The hiding generator is registered as the base after the last generator so that
-    `commit(elems, randomizer)` is a single device MSM (SURVEY.md App. A.2)."""
-    bases: "object"          # accumulation_b200.Bases: generators || hiding_generator
+    `commit(elems, randomizer)` is a single device MSM (SURVEY.md App. A.2); IpaPC's s, when given, follows it
+    (generators || h || s), so a zk opening's hiding_comm is one device MSM too."""
+    bases: "object"          # accumulation_b200.Bases: generators || hiding_generator [|| s]
     num_generators: int
+    s_index: Optional[int] = None
 
     @staticmethod
-    def new(ctx, curve: int, generators_xy, hiding_generator_xy=None, precompute: bool = False) -> "CommitterKey":
+    def new(ctx, curve: int, generators_xy, hiding_generator_xy=None, precompute: bool = False, s_xy=None) -> "CommitterKey":
         """precompute: also build the window table (once per key; trim / index time in the reference)"""
         gens = np.ascontiguousarray(generators_xy, dtype=np.uint64).reshape(-1, 8)
-        allb = gens if hiding_generator_xy is None else np.concatenate(
-            [gens, np.ascontiguousarray(hiding_generator_xy, dtype=np.uint64).reshape(1, 8)])
+        if s_xy is not None and hiding_generator_xy is None:
+            raise ValueError("CommitterKey.new: s follows the hiding generator h; pass both")
+        extra = [np.ascontiguousarray(p, dtype=np.uint64).reshape(1, 8) for p in (hiding_generator_xy, s_xy) if p is not None]
+        allb = np.concatenate([gens] + extra) if extra else gens
         bases = ctx.register_bases(curve, allb)
         if precompute:
             bases.precompute()
-        return CommitterKey(bases, gens.shape[0])
+        return CommitterKey(bases, gens.shape[0], None if s_xy is None else gens.shape[0] + 1)
 
     def supported_num_elems(self) -> int:   # src/hp_as/mod.rs:129,681
         return self.num_generators
@@ -82,22 +86,64 @@ def _int_to_fe(field: int, v: int) -> np.ndarray:
     return np.array([(w >> (64 * i)) & 0xFFFFFFFFFFFFFFFF for i in range(4)], dtype=np.uint64)
 
 
+def _canon(values) -> np.ndarray:
+    """canonical integers -> (n, 4) limbs"""
+    return np.array([[(v >> (64 * j)) & 0xFFFFFFFFFFFFFFFF for j in range(4)] for v in values], dtype=np.uint64).reshape(-1, 4)
+
+
+@dataclass
+class ZkHiding:
+    """What a zk opening (MakeZK::Enabled) adds to InnerProductArgPC.open: the random hiding polynomial (<= 2^k
+    coefficients from the caller's rng), its randomiser rho, the commitment C = (xy, inf) being opened with its randomness
+    r, and `alpha(hiding_comm) -> alpha`, the host sponge over (C, z, v, hiding_comm).  Montgomery limbs throughout."""
+    coeffs: "object"
+    rand: "object"
+    comm: tuple
+    comm_rand: "object"
+    alpha: Callable
+
+
 class InnerProductArgPC:
     """The parts of ark_poly_commit::ipa_pc::InnerProductArgPC that run the MSM."""
 
     @staticmethod
-    def open(ck: CommitterKey, combined_coeffs, point, h_prime_xy, round_challenge, log_d: Optional[int] = None, xi0=None):
+    def open(ck: CommitterKey, combined_coeffs, point, h_prime_xy, round_challenge, log_d: Optional[int] = None, xi0=None,
+             hiding: Optional["ZkHiding"] = None):
         """Core of open_individual_opening_challenges (SURVEY.md App. A.2; src/ipa_pc_as/mod.rs:454-462) after the
         host has combined the polynomials and derived h' = xi_0 * h (pass either the point h_prime_xy, or xi0 when h is the
         hiding generator of `ck`: faster, no separate scalar multiplication).  `round_challenge(prev_xi, l, r) -> xi` is the
         host sponge (Montgomery limbs in and out; prev_xi is None in the first round).
-        Returns (l_vec, r_vec, final_comm_key_xy, c, challenges)."""
+        hiding (MakeZK::Enabled, needs ck.s_index): before the first round the random polynomial is shifted to vanish at
+        the point and committed, alpha is squeezed from hiding_comm, P += alpha hiding' on the device and
+        C' = C + alpha hiding_comm - rand s with rand = r + alpha rho; xi0 (or h_prime_xy) may then be a callable of C'.
+        Returns (l_vec, r_vec, final_comm_key_xy, c, challenges), plus (hiding_comm, rand) when hiding is given."""
         from . import scalar_field
         ctx = ck.bases.ctx
         field = scalar_field(ck.curve)
         cf = np.ascontiguousarray(combined_coeffs, dtype=np.uint64).reshape(-1, 4)
         k = log_d if log_d is not None else max(cf.shape[0] - 1, 0).bit_length()
-        if xi0 is not None:      # h' = xi_0 * (hiding generator registered after the generators): no point needed
+        hiding_comm = rand = None
+        if hiding is not None:
+            if ck.s_index is None:
+                raise ValueError("InnerProductArgPC.open: a zk opening needs a key registered with s (CommitterKey.new(.., s_xy=))")
+            hp_now = None if callable(h_prime_xy) else h_prime_xy
+            sess = ctx.ipa_open_begin(ck.bases, cf, k, point, hp_now)
+            try:
+                hiding_comm = ctx.ipa_open_hide(sess, hiding.coeffs, ck.s_index, hiding.rand)
+                alpha = np.ascontiguousarray(hiding.alpha(hiding_comm), dtype=np.uint64).reshape(4)
+                ctx.ipa_open_hiding_challenge(sess, alpha)
+                rand = _int_to_fe(field, _fe_to_int(field, hiding.comm_rand) + _fe_to_int(field, alpha) * _fe_to_int(field, hiding.rand))
+                c_prime = InnerProductArgPC.hiding_commitment(ck, hiding.comm, hiding_comm, alpha, rand)
+                if callable(xi0):
+                    xi0 = xi0(c_prime)
+                if callable(h_prime_xy):
+                    raise ValueError("InnerProductArgPC.open: h' derived from C' goes in as xi0 (h' = xi_0 * h)")
+                if xi0 is not None:
+                    ctx.ipa_open_use_hiding_generator(sess, ck.num_generators, xi0)
+            except Exception:
+                InnerProductArgPC._release(ctx, sess)
+                raise
+        elif xi0 is not None:      # h' = xi_0 * (hiding generator registered after the generators): no point needed
             sess = ctx.ipa_open_begin(ck.bases, cf, k, point, None)
             ctx.ipa_open_use_hiding_generator(sess, ck.num_generators, xi0)
         else:
@@ -110,7 +156,29 @@ class InnerProductArgPC:
             l_vec.append(l); r_vec.append(r); challenges.append(xi)
             lr = ctx.ipa_open_fold_round(sess, xi)
         final_key, c = ctx.ipa_open_finish(sess)
+        if hiding is not None:
+            return l_vec, r_vec, final_key, c, challenges, hiding_comm, rand
         return l_vec, r_vec, final_key, c, challenges
+
+    @staticmethod
+    def _release(ctx, sess):
+        try:
+            ctx.ipa_open_finish(sess)       # finishing a session with rounds left releases it
+        except Exception:
+            pass
+
+    @staticmethod
+    def hiding_commitment(ck: CommitterKey, comm, hiding_comm, alpha, rand):
+        """C' = C + alpha hiding_comm - rand s, the commitment a zk opening proves against (upstream computes it on the
+        host before squeezing xi_0; here one 3-term device MSM) -> (xy, inf)"""
+        from . import scalar_field
+        f = scalar_field(ck.curve)
+        m = _MODULI[f]
+        s_xy = ck.bases.ctx.download_bases(ck.bases, ck.s_index, 1).reshape(8)
+        pts = np.array([np.asarray(comm[0], dtype=np.uint64), np.asarray(hiding_comm[0], dtype=np.uint64), s_xy])
+        inf = np.array([int(comm[1]), int(hiding_comm[1]), 0], dtype=np.uint8)
+        sc = _canon([1, _fe_to_int(f, alpha), (-_fe_to_int(f, rand)) % m])
+        return ck.bases.ctx.msm_oneshot(ck.curve, pts, sc, montgomery=False, infinity=inf)
 
     @staticmethod
     def cm_commit(comm_key: CommitterKey, scalars, hiding_generator_index: Optional[int] = None, randomizer=None):
@@ -121,31 +189,23 @@ class InnerProductArgPC:
         return comm_key.bases.ctx.commit(comm_key.bases, el, hiding_index=idx, randomizer_mont=randomizer)
 
     @staticmethod
-    def succinct_check_equation(ctx, curve: int, comm, point, value, l_vec, r_vec, round_challenges, h_prime_xy, final_comm_key_xy, c) -> bool:
+    def succinct_check_equation(ctx, curve: int, comm, point, value, l_vec, r_vec, round_challenges, h_prime_xy, final_comm_key_xy, c,
+                                hiding=None) -> bool:
         """Group equation of IpaPC::succinct_check (SURVEY.md App. A.2; src/ipa_pc_as/mod.rs:198-205) with the transcript
         values supplied by the host:  C + v h' + sum_i (xi_i^-1 l_i + xi_i r_i) == c final_comm_key + (h(z) c) h'.
         One 2k + 3 term MSM over unregistered points (accmsm_msm_oneshot) whose result must be the identity; the O(k)
-        scalar preparation (inverses, h(z)) is host arithmetic like in the reference.  comm = (xy, inf)."""
-        from . import scalar_field
-        f = scalar_field(curve)
-        m = _MODULI[f]
-        xis = [_fe_to_int(f, x) for x in np.asarray(round_challenges, dtype=np.uint64).reshape(-1, 4)]
-        k = len(xis)
-        z, v, cc = _fe_to_int(f, point), _fe_to_int(f, value), _fe_to_int(f, c)
-        hz = 1
-        for i, xi in enumerate(xis, start=1):
-            hz = hz * (1 + xi * pow(z, 1 << (k - i), m)) % m
-        bases = [np.asarray(comm[0], dtype=np.uint64)] + [np.asarray(p[0], dtype=np.uint64) for p in l_vec] + \
-                [np.asarray(p[0], dtype=np.uint64) for p in r_vec] + [np.asarray(h_prime_xy, dtype=np.uint64), np.asarray(final_comm_key_xy, dtype=np.uint64)]
-        inf = [int(comm[1])] + [int(p[1]) for p in l_vec] + [int(p[1]) for p in r_vec] + [0, 0]
-        scal = [1] + [pow(xi, -1, m) for xi in xis] + xis + [(v - hz * cc) % m, (-cc) % m]
-        sc = np.array([[(s_ >> (64 * j)) & 0xFFFFFFFFFFFFFFFF for j in range(4)] for s_ in scal], dtype=np.uint64)
-        _, res_inf = ctx.msm_oneshot(curve, np.array(bases), sc, montgomery=False, infinity=np.array(inf, dtype=np.uint8))
+        scalar preparation (inverses, h(z)) is host arithmetic like in the reference.  comm = (xy, inf).
+        hiding = (hiding_comm, alpha, rand, s_xy) of a zk proof: C becomes C' = C + alpha hiding_comm - rand s, two more
+        terms (2k + 5)."""
+        bases, inf, sc = InnerProductArgPC.succinct_check_terms(curve, comm, point, value, l_vec, r_vec, round_challenges, h_prime_xy,
+                                                                final_comm_key_xy, c, hiding)
+        _, res_inf = ctx.msm_oneshot(curve, bases, sc, montgomery=False, infinity=inf)
         return bool(res_inf)
 
     @staticmethod
-    def succinct_check_terms(curve: int, comm, point, value, l_vec, r_vec, round_challenges, h_prime_xy, final_comm_key_xy, c):
-        """(bases (2k + 3, 8), infinity flags, canonical scalars (2k + 3, 4)) of the equation above"""
+    def succinct_check_terms(curve: int, comm, point, value, l_vec, r_vec, round_challenges, h_prime_xy, final_comm_key_xy, c,
+                             hiding=None):
+        """(bases (2k + 3, 8), infinity flags, canonical scalars (2k + 3, 4)) of the equation above; 2k + 5 with hiding"""
         from . import scalar_field
         f = scalar_field(curve)
         m = _MODULI[f]
@@ -159,19 +219,33 @@ class InnerProductArgPC:
                 [np.asarray(p[0], dtype=np.uint64) for p in r_vec] + [np.asarray(h_prime_xy, dtype=np.uint64), np.asarray(final_comm_key_xy, dtype=np.uint64)]
         inf = [int(comm[1])] + [int(p[1]) for p in l_vec] + [int(p[1]) for p in r_vec] + [0, 0]
         scal = [1] + [pow(xi, -1, m) for xi in xis] + xis + [(v - hz * cc) % m, (-cc) % m]
-        sc = np.array([[(s_ >> (64 * j)) & 0xFFFFFFFFFFFFFFFF for j in range(4)] for s_ in scal], dtype=np.uint64)
-        return np.array(bases), np.array(inf, dtype=np.uint8), sc
+        if hiding is not None:
+            hiding_comm, alpha, rand, s_xy = hiding
+            bases += [np.asarray(hiding_comm[0], dtype=np.uint64), np.asarray(s_xy, dtype=np.uint64).reshape(8)]
+            inf += [int(hiding_comm[1]), 0]
+            scal += [_fe_to_int(f, alpha), (-_fe_to_int(f, rand)) % m]
+        return np.array(bases), np.array(inf, dtype=np.uint8), _canon(scal)
 
     @staticmethod
     def succinct_check_equations(ctx, curve: int, instances) -> list:
         """The equations of ALL inputs and accumulators of one prove / verify (the loops at src/ipa_pc_as/mod.rs:262-270 and
         :625-640 call succinct_check once per instance) as ONE batched call (accmsm_msm_oneshot_batch): `instances` is a list
-        of argument tuples of succinct_check_equation (without ctx and curve), all of the same degree."""
+        of argument tuples of succinct_check_equation (without ctx and curve), all of the same degree.  zk instances (with
+        the hiding tuple) and others mix: the others are padded with two (identity, 0) terms."""
         terms = [InnerProductArgPC.succinct_check_terms(curve, *inst) for inst in instances]
         if not terms:
             return []
-        _, inf = ctx.msm_oneshot_batch(curve, np.stack([t[0] for t in terms]), np.stack([t[2] for t in terms]), montgomery=False,
-                                       infinity=np.stack([t[1] for t in terms]))
+        width = max(t[0].shape[0] for t in terms)
+        padded = []
+        for b, i, sc in terms:
+            pad = width - b.shape[0]
+            if pad:
+                b = np.concatenate([b, np.repeat(b[:1], pad, axis=0)])
+                i = np.concatenate([i, np.ones(pad, dtype=np.uint8)])
+                sc = np.concatenate([sc, np.zeros((pad, 4), dtype=np.uint64)])
+            padded.append((b, i, sc))
+        _, inf = ctx.msm_oneshot_batch(curve, np.stack([t[0] for t in padded]), np.stack([t[2] for t in padded]), montgomery=False,
+                                       infinity=np.stack([t[1] for t in padded]))
         return [bool(x) for x in inf]
 
     @staticmethod

@@ -236,6 +236,19 @@ int accmsm_ipa_open_fold(accmsm_ctx *ctx, uint64_t session, const uint64_t xi_mo
 int accmsm_ipa_open_fold_round(accmsm_ctx *ctx, uint64_t session, const uint64_t xi_mont[4], uint64_t l_xy[8], uint8_t *l_inf,
                                uint64_t r_xy[8], uint8_t *r_inf, int *done);
 int accmsm_ipa_open_finish(accmsm_ctx *ctx, uint64_t session, uint64_t final_key_xy[8], uint64_t c_mont[4]);
+/* Zero-knowledge opening (MakeZK::Enabled; SURVEY.md 3.2, App. A.2 hiding_comm / rand).  Between begin (or
+ * begin_combined) and the first round, in this order:
+ *     hide(hiding, s_index, rho) -> hiding_comm;  alpha = sponge(C, z, v, hiding_comm);  hiding_challenge(alpha)
+ *     C' = C + alpha hiding_comm - (r + alpha rho) s on the host, xi_0 from C', then the rounds as above
+ * hide: uploads the caller's random polynomial (n_hiding <= 2^k coefficients, zero padded), evaluates it at the point and
+ *       subtracts the value from coefficient 0 (the polynomial then vanishes there, so eval_out of begin_combined stays
+ *       P'(z)), and returns hiding_comm = cm_commit(key[0, 2^k), hiding') + rho key[s_index] from one MSM pass.
+ * hiding_challenge: coeffs += alpha hiding' (enqueued only).
+ * ACCMSM_E_ARG: hide after the first round or twice, hiding_challenge without hide or twice, a round / fold / finish of a
+ * hidden session before its hiding_challenge, n_hiding > 2^k, s_index beyond the key, a session begun with log_shards > 0. */
+int accmsm_ipa_open_hide(accmsm_ctx *ctx, uint64_t session, const uint64_t *hiding_coeffs_mont, size_t n_hiding, size_t s_index,
+                         const uint64_t hiding_rand_mont[4], uint64_t hiding_comm_xy[8], uint8_t *hiding_comm_inf);
+int accmsm_ipa_open_hiding_challenge(accmsm_ctx *ctx, uint64_t session, const uint64_t alpha_mont[4]);
 
 /* Multi-GPU opening (SURVEY.md 8e, "IPA open folding"): the key, the coefficients and the z-vector are sharded
  * CYCLICALLY, shard g of G = 2^log_shards owns the indices i with i mod G == g, so the fold partners i and i + n/2 stay
