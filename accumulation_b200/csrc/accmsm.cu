@@ -397,8 +397,10 @@ int launch_scan(accmsm_ctx *ctx, const uint32_t *counts, uint32_t nkeys, uint32_
 }
 
 constexpr size_t SORT_SMEM_OPT_IN = 220 * 1024;      // dynamic shared memory the sort kernels may use (227 KB per CTA minus their static part)
+// both tile passes: the count pass asks for 2 nparts words, more than the 48 KB default once nparts > 6144
 template <class Src> bool sort_opt_in() {
-    return cudaFuncSetAttribute(k_sort_tiles<Src, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)SORT_SMEM_OPT_IN) == cudaSuccess;
+    return cudaFuncSetAttribute(k_sort_tiles<Src, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)SORT_SMEM_OPT_IN) == cudaSuccess &&
+           cudaFuncSetAttribute(k_sort_tiles<Src, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)SORT_SMEM_OPT_IN) == cudaSuccess;
 }
 
 // ---- the MSM pipeline in two stages ---------------------------------------------------------------------------------
@@ -458,6 +460,7 @@ int msm_accumulate(accmsm_ctx *ctx, const Bases &B, const MsmJobs &jobs, size_t 
         trace_point(ctx, st, "  sort begins");
         CU(ctx, cudaMemsetAsync(max_part, 0, sizeof(uint32_t), st));
         k_sort_tiles<Src, false><<<pl.ntiles, SORT_THREADS, smem0, st>>>(src, sh, B.d_inf, pl, 0u, pl.tiles_per_job, tile_count, tile_hist, nullptr, nullptr, gate);
+        CU(ctx, cudaGetLastError());      // a refused count launch leaves tile_count unwritten: nothing below may read it
         mark(ctx, ST_SCAN, st);
         k_sort_tile_scan<<<(pl.nparts + TS_PARTS - 1) / TS_PARTS, TS_PARTS * TS_SEGS, 0, st>>>(tile_count, pl.ntiles, pl.nparts, ctx->sort_part_count.p, max_part);
         ctx->launches += 2;
