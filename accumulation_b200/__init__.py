@@ -451,6 +451,36 @@ class Context:
                                                        None if vecs is None else self._ptrs(vecs), _p(out), _p(oinf)), "csr_matvec_commit")
         return vecs, out, oinf
 
+    def nark_prove_zk(self, bases: "Bases", csr: int, n_rows: int, inp, wit, r, blinders, hiding_index: int = 0, want_vecs: bool = True):
+        """zk R1CSNark::prove first message: z_M, r_M, cross, rr and their 8 commitments (blinders: 8 x 4 in the order
+        A, B, C, rA, rB, rC, 1, 2) in one vector launch and one pass -> (vecs | None, xy (8, 8), inf (8,))"""
+        inp, wit, r = _u64(inp).reshape(-1, 4), _u64(wit).reshape(-1, 4), _u64(r).reshape(-1, 4)
+        bl = _u64(blinders).reshape(8, 4)
+        vecs = [np.empty((n_rows, 4), dtype=np.uint64) for _ in range(8)] if want_vecs else None
+        out = np.empty((8, 8), dtype=np.uint64)
+        oinf = np.zeros(8, dtype=np.uint8)
+        self._check(self._lib.accmsm_nark_prove_zk(self._h, C.c_uint64(bases.handle), C.c_uint64(csr), _p(inp), C.c_size_t(inp.shape[0]),
+                                                   _p(wit), C.c_size_t(wit.shape[0]), _p(r), C.c_size_t(hiding_index), _p(bl),
+                                                   None if vecs is None else self._ptrs(vecs), _p(out), _p(oinf)), "nark_prove_zk")
+        return vecs, out, oinf
+
+    def nark_verify(self, bases: "Bases", csr: int, n_rows: int, inp, blinded_wit, expected_xy, expected_inf, hiding_index: int = 0,
+                    sigmas=None, want_vecs: bool = False):
+        """R1CSNark::verify: t_M = M (input || w'), Commit(t_M, sigma_M) and Commit(t_A o t_B, sigma_o) in one vector launch and
+        one pass, compared with the 4 expected points -> (accept, [t_A, t_B, t_C] | None, xy (4, 8), inf (4,))"""
+        inp, wit = _u64(inp).reshape(-1, 4), _u64(blinded_wit).reshape(-1, 4)
+        exp = _u64(expected_xy).reshape(4, 8)
+        einf = np.ascontiguousarray(expected_inf, dtype=np.uint8).reshape(4)
+        sg = None if sigmas is None else _u64(sigmas).reshape(4, 4)
+        vecs = [np.empty((n_rows, 4), dtype=np.uint64) for _ in range(3)] if want_vecs else None
+        out = np.empty((4, 8), dtype=np.uint64)
+        oinf = np.zeros(4, dtype=np.uint8)
+        acc = C.c_int(0)
+        self._check(self._lib.accmsm_nark_verify(self._h, C.c_uint64(bases.handle), C.c_uint64(csr), _p(inp), C.c_size_t(inp.shape[0]),
+                                                 _p(wit), C.c_size_t(wit.shape[0]), C.c_size_t(hiding_index), _p(sg), _p(exp), _p(einf),
+                                                 C.byref(acc), _p(out), _p(oinf), None if vecs is None else self._ptrs(vecs)), "nark_verify")
+        return bool(acc.value), vecs, out, oinf
+
     # ---- field-vector kernels
     def compute_coeffs(self, field: int, challenges_mont):
         ch = _u64(challenges_mont).reshape(-1, 4)
@@ -559,8 +589,8 @@ class Bases:
 
 
 from .mirror import (  # noqa: E402
-    ASForHadamardProducts, CommitterKey, InnerProductArgPC, PedersenCommitment, R1CSNark, SuccinctCheckPolynomial, ZkHiding, matrix_vec_mul,
+    ASForHadamardProducts, CommitterKey, InnerProductArgPC, NarkProof, PedersenCommitment, R1CSNark, SuccinctCheckPolynomial, ZkHiding, matrix_vec_mul,
 )
 
 __all__ = ["Context", "Bases", "pinned_array", "release_pinned", "AccmsmError", "PALLAS", "VESTA", "FP", "FQ", "scalar_field", "PedersenCommitment",
-           "CommitterKey", "InnerProductArgPC", "SuccinctCheckPolynomial", "ZkHiding", "ASForHadamardProducts", "R1CSNark", "matrix_vec_mul"]
+           "CommitterKey", "InnerProductArgPC", "SuccinctCheckPolynomial", "ZkHiding", "ASForHadamardProducts", "R1CSNark", "NarkProof", "matrix_vec_mul"]

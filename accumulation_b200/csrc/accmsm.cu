@@ -979,6 +979,9 @@ int group_release_csr(accmsm_ctx *g, uint64_t handle);
 int group_csr_matvec_commit(accmsm_ctx *g, uint64_t key_handle, uint64_t csr_handle, const uint64_t *input, size_t n_input,
                             const uint64_t *witness, size_t n_witness, size_t hiding_index, const uint64_t *blinders_mont,
                             uint64_t *const *out_vecs, uint64_t *out_xy, uint8_t *out_inf);
+int group_nark(accmsm_ctx *g, bool prove, uint64_t key_handle, uint64_t csr_handle, const uint64_t *input, size_t n_input,
+               const uint64_t *witness, size_t n_witness, const uint64_t *r, size_t hiding_index, const uint64_t *tails_mont,
+               uint64_t *const *out_vecs, uint64_t *out_xy, uint8_t *out_inf);
 int group_open_key(accmsm_ctx *g, uint64_t handle, uint64_t *kid0_handle);     // full key on child 0 for IpaPC::open sessions
 // IpaPC::open sessions sharded cyclically across the children of a group (multi_api.inc).  GROUP_IPA_UNSHARDED: the
 // opening is too small to shard / the id is not a sharded session, and child 0 serves the call as before.

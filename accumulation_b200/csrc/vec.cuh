@@ -201,4 +201,53 @@ __global__ void __launch_bounds__(256) k_csr_matvec(CsrMats mats, uint32_t n_row
     store_fe(mats.out[mi] + (size_t)r * 32, acc);
 }
 
+// R1CSNark rows (src/r1cs_nark_as/r1cs_nark/mod.rs:183-261 prove, :335-419 verify): one thread per constraint row walks row r
+// of A, B and C once.  Every (col, coeff) is loaded once and feeds the z-sum over input || witness and, with ZK, the r-sum
+// over 0 || r (input columns add nothing to it).  The products are formed in registers and every result goes straight to
+// row j of the pass's scalar rows (out + j * row_stride):
+//   ZK:  z_A, z_B, z_C, r_A, r_B, r_C, cross = z_A r_B + z_B r_A, rr = r_A r_B
+//   !ZK: t_A, t_B, t_C, t_A t_B
+template <int FIELD, bool ZK>
+__global__ void __launch_bounds__(256) k_nark_rows(CsrMats mats, uint32_t n_rows, const uint8_t *__restrict__ input, uint32_t n_input,
+                                                    const uint8_t *__restrict__ witness, const uint8_t *__restrict__ rvec,
+                                                    uint8_t *__restrict__ out, size_t row_stride) {
+    using F = Fp<FIELD>;
+    uint32_t r = blockIdx.x * blockDim.x + threadIdx.x;
+    if (r >= n_rows) return;
+    const fe_t one = F::one();
+    fe_t za = F::zero(), zb = F::zero(), ra = F::zero(), rb = F::zero();
+#pragma unroll
+    for (int mi = 0; mi < 3; mi++) {
+        fe_t zs = F::zero(), rs = F::zero();
+        const uint32_t e0 = mats.row_ptr[mi][r], e1 = mats.row_ptr[mi][r + 1];
+        for (uint32_t e = e0; e < e1; e++) {
+            const uint32_t col = mats.cols[mi][e];
+            const fe_t cf = load_fe_nc(mats.coeffs[mi] + (size_t)e * 32);
+            const bool unit = F::eq(cf, one);          // coeff.is_one() fast path (:459)
+            if (col < n_input) {
+                const fe_t z = load_fe(input + (size_t)col * 32);
+                zs = F::add(zs, unit ? z : F::mul(z, cf));
+            } else {
+                const size_t w = (size_t)(col - n_input) * 32;
+                const fe_t z = load_fe(witness + w);
+                zs = F::add(zs, unit ? z : F::mul(z, cf));
+                if (ZK) {
+                    const fe_t rv = load_fe(rvec + w);
+                    rs = F::add(rs, unit ? rv : F::mul(rv, cf));
+                }
+            }
+        }
+        store_fe(out + (size_t)mi * row_stride + (size_t)r * 32, zs);
+        if (ZK) store_fe(out + (size_t)(3 + mi) * row_stride + (size_t)r * 32, rs);
+        if (mi == 0) { za = zs; ra = rs; }
+        if (mi == 1) { zb = zs; rb = rs; }
+    }
+    if (ZK) {
+        store_fe(out + (size_t)6 * row_stride + (size_t)r * 32, F::add(F::mul(za, rb), F::mul(zb, ra)));
+        store_fe(out + (size_t)7 * row_stride + (size_t)r * 32, F::mul(ra, rb));
+    } else {
+        store_fe(out + (size_t)3 * row_stride + (size_t)r * 32, F::mul(za, zb));
+    }
+}
+
 }  // namespace accmsm

@@ -10,8 +10,9 @@
 //   ipa_pc::SuccinctCheckPolynomial(Vec<F>)::compute_coeffs            SuccinctCheckPolynomial::compute_coeffs
 //   hp_as: compute_hp, compute_t_vecs, combine_vectors, scale_vector,  ASForHadamardProducts::...
 //          compute_product_poly_comm, decide   (src/hp_as/mod.rs:278-512, 894-925)
-//   r1cs_nark: Matrix<F> = Vec<Vec<(F, usize)>>, matrix_vec_mul        r1cs_nark::{Matrix, matrix_vec_mul, IndexMatrices}
-//                                        (src/r1cs_nark_as/r1cs_nark/mod.rs:443-462)
+//   r1cs_nark: Matrix<F> = Vec<Vec<(F, usize)>>, matrix_vec_mul,       r1cs_nark::{Matrix, matrix_vec_mul, IndexMatrices}
+//              R1CSNark::prove (zk first message) / verify             IndexMatrices::{matvec_commit, prove_zk, verify}
+//                                        (src/r1cs_nark_as/r1cs_nark/mod.rs:183-419, 443-462)
 // Every call computes on the GPU; there is no CPU path.  ark's commit is infallible -> failures throw AccmsmError
 // (the Rust wrapper panics / maps to PCError at the same places).
 #pragma once
@@ -383,6 +384,7 @@ public:
         ck.ctx()->check(accmsm_register_csr(ck.ctx()->raw(), scalar_field(ck.curve()), 3, rp, cl, cf, n_rows_, &handle_), "register_csr");
     }
     ~IndexMatrices() { accmsm_release_csr(ck_.ctx()->raw(), handle_); }
+    uint64_t handle() const { return handle_; }
     // z_M = M (input || witness), comm_M = Commit(z_M, blinder_M)   (prove :183-185 + :216-218; decide src/r1cs_nark_as/mod.rs:1052-1097)
     std::pair<std::vector<std::vector<Fe>>, std::vector<Affine>> matvec_commit(const std::vector<Fe> &input, const std::vector<Fe> &witness,
                                                                               const std::optional<std::array<Fe, 3>> &blinders = std::nullopt) const {
@@ -396,6 +398,41 @@ public:
         std::vector<Affine> comms;
         for (int m = 0; m < 3; m++) comms.push_back(affine_from(xy + 8 * m, inf[m]));
         return {vecs, comms};
+    }
+    // zk prove first message (prove :183-261): Commit(z_M, blinder_M), Commit(r_M, rblinder_M), Commit(cross, blinder_1),
+    // Commit(rr, blinder_2) with z_M = M (input || witness), r_M = M (0 || r), in ONE library call (one vector launch, one
+    // pass).  blinders and the result in the order A, B, C, rA, rB, rC, 1, 2.  The caller squeezes gamma from the result,
+    // forms w' = w + gamma r (ASForHadamardProducts::combine_vectors) and the sigmas, as upstream.
+    std::vector<Affine> prove_zk(const std::vector<Fe> &input, const std::vector<Fe> &witness, const std::vector<Fe> &r,
+                                 const std::array<Fe, 8> &blinders) const {
+        if (!ck_.has_hiding()) throw AccmsmError("prove_zk: the key has no hiding generator");
+        if (r.size() != witness.size()) throw AccmsmError("prove_zk: r must be as long as the witness");
+        uint64_t xy[64]; uint8_t inf[8];
+        ck_.ctx()->check(accmsm_nark_prove_zk(ck_.ctx()->raw(), ck_.handle(), handle_, input.empty() ? nullptr : input[0].data(), input.size(),
+                                              witness.empty() ? nullptr : witness[0].data(), witness.size(), r.empty() ? nullptr : r[0].data(),
+                                              ck_.hiding_index(), blinders[0].data(), nullptr, xy, inf), "nark_prove_zk");
+        std::vector<Affine> first;
+        for (int j = 0; j < 8; j++) first.push_back(affine_from(xy + 8 * j, inf[j]));
+        return first;
+    }
+    // verify (:335-419): accept iff Commit(t_M, sigma_M) == expected[M] and Commit(t_A o t_B, sigma_o) == expected[3], with
+    // t_M = M (input || blinded_witness), in ONE library call.  expected: comm_M + gamma comm_rM and comm_C + gamma comm_1 +
+    // gamma^2 comm_2, or without zk (sigmas = nullopt) comm_A, comm_B, comm_C, comm_C.  t_vecs (nullable) receives t_A, t_B, t_C.
+    bool verify(const std::vector<Fe> &input, const std::vector<Fe> &blinded_witness, const std::array<Affine, 4> &expected,
+                const std::optional<std::array<Fe, 4>> &sigmas = std::nullopt, std::vector<std::vector<Fe>> *t_vecs = nullptr) const {
+        uint64_t exp[32]; uint8_t einf[4];
+        for (int j = 0; j < 4; j++) { affine_to(expected[j], exp + 8 * j); einf[j] = expected[j].infinity; }
+        uint64_t *op[3] = {nullptr, nullptr, nullptr};
+        if (t_vecs) {
+            t_vecs->assign(3, std::vector<Fe>(n_rows_));
+            if (n_rows_) for (int m = 0; m < 3; m++) op[m] = (*t_vecs)[m][0].data();
+        }
+        int accept = 0;
+        ck_.ctx()->check(accmsm_nark_verify(ck_.ctx()->raw(), ck_.handle(), handle_, input.empty() ? nullptr : input[0].data(), input.size(),
+                                            blinded_witness.empty() ? nullptr : blinded_witness[0].data(), blinded_witness.size(),
+                                            ck_.hiding_index(), sigmas ? (*sigmas)[0].data() : nullptr, exp, einf, &accept, nullptr, nullptr,
+                                            t_vecs ? op : nullptr), "nark_verify");
+        return accept != 0;
     }
 private:
     const CommitterKey &ck_;

@@ -313,8 +313,18 @@ class ASForHadamardProducts:
         return ok
 
 
+@dataclass
+class NarkProof:
+    """r1cs_nark::Proof (src/r1cs_nark_as/r1cs_nark/data_structures.rs): first_msg = [comm_a, comm_b, comm_c] without zk, or
+    [comm_a, comm_b, comm_c, comm_r_a, comm_r_b, comm_r_c, comm_1, comm_2] with it, as (xy, inf); blinded_witness = w (no zk)
+    or w' = w + gamma r; sigmas = (sigma_a, sigma_b, sigma_c, sigma_o) as (4, 4) Montgomery limbs, None without zk."""
+    first_msg: list
+    blinded_witness: "object"
+    sigmas: "object" = None
+
+
 class R1CSNark:
-    """The mat-vec + commitment steps of src/r1cs_nark_as/r1cs_nark/mod.rs (prove :183-218, verify :356-389) and of
+    """The mat-vec + commitment steps of src/r1cs_nark_as/r1cs_nark/mod.rs (prove :183-316, verify :335-419) and of
     ASForR1CSNark::decide (src/r1cs_nark_as/mod.rs:1052-1097) with the index matrices registered once."""
 
     def __init__(self, ck: CommitterKey, matrices):
@@ -329,6 +339,50 @@ class R1CSNark:
         vecs, xy, inf = self.ck.bases.ctx.csr_matvec_commit(self.ck.bases, self.csr, self.n_mats, self.n_rows, inp, wit,
                                                              hiding_index=self.ck.num_generators, blinders=blinders)
         return vecs, [(xy[i], int(inf[i])) for i in range(self.n_mats)]
+
+    def prove(self, inp, wit, gamma_fn: Callable, zk=None) -> NarkProof:
+        """R1CSNark::prove (:183-316).  zk = (r, blinders): the random witness-length vector and the 8 blinders in the order
+        A, B, C, rA, rB, rC, 1, 2 (the caller's rng); gamma_fn(first_msg) -> gamma is the host sponge over the first message.
+        Without zk: one matvec_commit.  With zk: one nark_prove_zk call (one vector launch + one 8-job pass), then
+        w' = w + gamma r on the device and the sigmas on the host."""
+        from . import scalar_field
+        if zk is None:
+            _, comms = self.matvec_commit(inp, wit)
+            return NarkProof(comms, np.ascontiguousarray(wit, dtype=np.uint64).reshape(-1, 4), None)
+        ctx, f = self.ck.bases.ctx, scalar_field(self.ck.curve)
+        r, blinders = zk
+        _, xy, inf = ctx.nark_prove_zk(self.ck.bases, self.csr, self.n_rows, inp, wit, r, blinders, hiding_index=self.ck.num_generators,
+                                       want_vecs=False)
+        first = [(xy[i], int(inf[i])) for i in range(8)]
+        gamma = np.ascontiguousarray(gamma_fn(first), dtype=np.uint64).reshape(4)
+        w = np.ascontiguousarray(wit, dtype=np.uint64).reshape(-1, 4)
+        w_prime = ctx.lincomb(f, [r], gamma.reshape(1, 4), hiding=w) if w.shape[0] else w
+        m, g = _MODULI[f], _fe_to_int(f, gamma)
+        b = [_fe_to_int(f, x) for x in np.asarray(blinders, dtype=np.uint64).reshape(8, 4)]
+        sig = [b[i] + g * b[3 + i] for i in range(3)] + [b[2] + g * b[6] + g * g % m * b[7]]
+        return NarkProof(first, w_prime, np.array([_int_to_fe(f, s) for s in sig]))
+
+    def verify(self, inp, proof: NarkProof, gamma=None) -> bool:
+        """R1CSNark::verify (:335-419).  With zk the four left-hand sides comm_M + gamma comm_rM and comm_C + gamma comm_1 +
+        gamma^2 comm_2 come from ONE msm_oneshot_batch (4 equations x 3 terms, the 2-term ones padded with (identity, 0));
+        then one nark_verify call: t_M = M (input || w'), the 4 commitments in one pass, and the comparison."""
+        from . import scalar_field
+        ctx, f = self.ck.bases.ctx, scalar_field(self.ck.curve)
+        fm = proof.first_msg
+        if proof.sigmas is None:
+            lhs = [fm[0], fm[1], fm[2], fm[2]]
+        else:
+            m, g = _MODULI[f], _fe_to_int(f, gamma)
+            eqs = [[(fm[i], 1), (fm[3 + i], g), (fm[i], None)] for i in range(3)] + [[(fm[2], 1), (fm[6], g), (fm[7], g * g % m)]]
+            pts = np.array([[np.asarray(p[0], dtype=np.uint64) for p, _ in eq] for eq in eqs])
+            infs = np.array([[1 if s is None else int(p[1]) for p, s in eq] for eq in eqs], dtype=np.uint8)
+            sc = np.stack([_canon([0 if s is None else s for _, s in eq]) for eq in eqs])
+            xy, inf = ctx.msm_oneshot_batch(self.ck.curve, pts, sc, montgomery=False, infinity=infs)
+            lhs = [(xy[i], int(inf[i])) for i in range(4)]
+        ok, _, _, _ = ctx.nark_verify(self.ck.bases, self.csr, self.n_rows, inp, proof.blinded_witness,
+                                      np.array([np.asarray(p[0], dtype=np.uint64) for p in lhs]), [p[1] for p in lhs],
+                                      hiding_index=self.ck.num_generators, sigmas=proof.sigmas)
+        return ok
 
     def release(self):
         self.ck.bases.ctx.release_csr(self.csr)

@@ -342,6 +342,28 @@ int accmsm_csr_matvec_commit_partial_dev(accmsm_ctx *ctx, uint64_t key_handle, u
                                          const uint64_t *witness, size_t n_witness, size_t hiding_index, const uint64_t *blinders_mont,
                                          uint64_t *const *out_vecs, void *d_out_partials);
 
+/* zk R1CSNark::prove first message (src/r1cs_nark_as/r1cs_nark/mod.rs:183-261): z_M = M (x||w), r_M = M (0||r),
+ * cross = z_A o r_B + z_B o r_A, rr = r_A o r_B, and the 8 commitments in ONE pass.  csr_handle must hold 3 matrices.
+ * r: n_witness x 4.  blinders: 8 x 4, in the order A, B, C, rA, rB, rC, 1, 2 (required).
+ * out_xy: 8 x 8, out_inf: 8, in the same order.  out_vecs: NULL, or 8 nullable pointers (n_rows x 4).
+ * The prover then squeezes gamma and forms w' = w + gamma r with accmsm_vec_lincomb (hiding = w, vecs = [r], ch = [gamma]),
+ * sigma_M = blinder_M + gamma rblinder_M and sigma_o = blinder_C + gamma blinder_1 + gamma^2 blinder_2 (:262-316).
+ * One pass of 8 jobs over n_rows + 1 pairs needs 8 x windows x (n_rows + 1) < 2^31: n_rows < ~2^24 at c = 20.
+ * The non-zk prove is accmsm_csr_matvec_commit. */
+int accmsm_nark_prove_zk(accmsm_ctx *ctx, uint64_t key_handle, uint64_t csr_handle, const uint64_t *input, size_t n_input,
+                         const uint64_t *witness, size_t n_witness, const uint64_t *r, size_t hiding_index,
+                         const uint64_t *blinders_mont, uint64_t *const *out_vecs, uint64_t *out_xy, uint8_t *out_inf);
+/* R1CSNark::verify (:335-419): t_M = M (x||w'), then Commit(t_A, s_A), Commit(t_B, s_B), Commit(t_C, s_C) and
+ * Commit(t_A o t_B, s_o) in ONE pass, compared with expected_xy / expected_inf (4 points, which the caller combines from the
+ * proof: comm_M + gamma comm_rM and comm_C + gamma comm_1 + gamma^2 comm_2; without zk comm_A, comm_B, comm_C, comm_C).
+ * sigmas: 4 x 4, or NULL without zk.  out_vecs: NULL, or 3 nullable pointers (t_A, t_B, t_C; t_A and t_B are also the
+ * hp witnesses of ASForR1CSNark::compute_hp_input_witnesses, src/r1cs_nark_as/mod.rs).  out_xy / out_inf nullable.
+ * One pass of 4 jobs: n_rows < ~2^25 at c = 20. */
+int accmsm_nark_verify(accmsm_ctx *ctx, uint64_t key_handle, uint64_t csr_handle, const uint64_t *input, size_t n_input,
+                       const uint64_t *blinded_witness, size_t n_witness, size_t hiding_index, const uint64_t *sigmas_mont,
+                       const uint64_t *expected_xy, const uint8_t *expected_inf, int *accept, uint64_t *out_xy,
+                       uint8_t *out_inf, uint64_t *const *out_vecs);
+
 #ifdef __cplusplus
 }
 #endif
