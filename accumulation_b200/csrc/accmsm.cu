@@ -910,6 +910,11 @@ template <int CURVE> void launch_identity_partials(accmsm_ctx *ctx, xyzz_t *d_ou
     k_finish<CURVE><<<k, 32, 0, st>>>(nullptr, 0, 1, nullptr, 0, d_out, nullptr);
     ctx->launches++;
 }
+int launch_identity_partials(accmsm_ctx *ctx, int curve, xyzz_t *d_out, uint32_t k, cudaStream_t st) {
+    if (curve == 0) launch_identity_partials<0>(ctx, d_out, k, st); else launch_identity_partials<1>(ctx, d_out, k, st);
+    CU(ctx, cudaGetLastError());
+    return ACCMSM_OK;
+}
 
 // k scalar vectors from the host (k x n x 32 B) against bases [offset, offset + n), optional last pair
 // (base tail_index, tail[j]) per vector, as ONE pass per MAX_JOBS vectors; un-normalised sums -> d_partials[0..k)
@@ -921,7 +926,7 @@ int msm_rows_host(accmsm_ctx *ctx, const Bases &B, size_t offset, size_t n, size
     const size_t n_eff = n + (tail ? 1 : 0), row = n_eff * 32;
     clear_marks(ctx);
     if (n_eff == 0) {
-        if (d_partials) { if (B.curve == 0) launch_identity_partials<0>(ctx, d_partials, (uint32_t)k, st); else launch_identity_partials<1>(ctx, d_partials, (uint32_t)k, st); }
+        if (d_partials) { int rc = launch_identity_partials(ctx, B.curve, d_partials, (uint32_t)k, st); if (rc) return rc; }
         if (out_xy) for (size_t j = 0; j < k; j++) write_identity(ctx, B.curve, out_xy + 8 * j, out_inf + j);
         CU(ctx, cudaStreamSynchronize(st));
         return ACCMSM_OK;
@@ -976,12 +981,9 @@ int group_hp_product_poly_comm(accmsm_ctx *g, uint64_t handle, const uint64_t *c
 int group_register_csr(accmsm_ctx *g, int field, int n_mats, const uint32_t *const *row_ptr, const uint32_t *const *cols,
                        const uint64_t *const *coeffs_mont, size_t n_rows, uint64_t *handle);
 int group_release_csr(accmsm_ctx *g, uint64_t handle);
-int group_csr_matvec_commit(accmsm_ctx *g, uint64_t key_handle, uint64_t csr_handle, const uint64_t *input, size_t n_input,
-                            const uint64_t *witness, size_t n_witness, size_t hiding_index, const uint64_t *blinders_mont,
-                            uint64_t *const *out_vecs, uint64_t *out_xy, uint8_t *out_inf);
-int group_nark(accmsm_ctx *g, bool prove, uint64_t key_handle, uint64_t csr_handle, const uint64_t *input, size_t n_input,
-               const uint64_t *witness, size_t n_witness, const uint64_t *r, size_t hiding_index, const uint64_t *tails_mont,
-               uint64_t *const *out_vecs, uint64_t *out_xy, uint8_t *out_inf);
+template <class F>
+int group_csr_pass(accmsm_ctx *g, const std::string &what, uint64_t key_handle, uint64_t csr_handle, size_t n_z, size_t hiding_index,
+                   const uint64_t *tails_mont, size_t m, size_t n_vecs, uint64_t *const *out_vecs, uint64_t *out_xy, uint8_t *out_inf, F run);
 int group_open_key(accmsm_ctx *g, uint64_t handle, uint64_t *kid0_handle);     // full key on child 0 for IpaPC::open sessions
 // IpaPC::open sessions sharded cyclically across the children of a group (multi_api.inc).  GROUP_IPA_UNSHARDED: the
 // opening is too small to shard / the id is not a sharded session, and child 0 serves the call as before.
@@ -998,6 +1000,14 @@ int group_ipa_hide(accmsm_ctx *g, uint64_t session, const uint64_t *hiding_mont,
                    const uint64_t rho_mont[4], uint64_t comm_xy[8], uint8_t *comm_inf);
 int group_ipa_hiding_challenge(accmsm_ctx *g, uint64_t session, const uint64_t alpha_mont[4]);
 inline bool is_group(const accmsm_ctx *ctx) { return ctx && !ctx->kids.empty(); }
+// the result of a call a group forwarded to child 0, with child 0's error message
+inline int group_fwd0(accmsm_ctx *g, int rc) { if (rc) g->last_error = g->kids[0]->last_error; return rc; }
+// fn(child 0, handle of the whole key on child 0), forwarded: IpaPC::open sessions too small to shard
+template <class F> int group_fwd0_open_key(accmsm_ctx *g, uint64_t handle, F fn) {
+    uint64_t h0 = 0;
+    { std::lock_guard<std::mutex> lock(g->mu); int rc = group_open_key(g, handle, &h0); if (rc) return rc; }
+    return group_fwd0(g, fn(g->kids[0], h0));
+}
 #define GROUP_NO_DEV(ctx, name) do { if (is_group(ctx)) return fail_arg(ctx, name ": device-pointer entry points need a single-device ctx (accmsm_device_ctx)"); } while (0)
 
 // =====================================================================================================
