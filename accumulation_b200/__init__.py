@@ -481,6 +481,26 @@ class Context:
                                                  C.byref(acc), _p(out), _p(oinf), None if vecs is None else self._ptrs(vecs)), "nark_verify")
         return bool(acc.value), vecs, out, oinf
 
+    def nark_as_decide(self, bases: "Bases", csr: int, inp, wit, hp_a, hp_b, expected_xy, expected_inf, hiding_index: int = 0,
+                       sigmas=None, hp_randomness=None):
+        """ASForR1CSNark::decide: t_M = M (input || w*), Commit(t_M, sigma_M*), Commit(a*, r1*), Commit(b*, r2*) and
+        Commit(a* o b*, r3*) in one vector launch and one 6-job pass, compared with the 6 expected points (comm_A*, comm_B*,
+        comm_C*, C1*, C2*, C3*) -> (accept, xy (6, 8), inf (6,))"""
+        inp, wit = _u64(inp).reshape(-1, 4), _u64(wit).reshape(-1, 4)
+        a, b = _u64(hp_a).reshape(-1, 4), _u64(hp_b).reshape(-1, 4)
+        exp = _u64(expected_xy).reshape(6, 8)
+        einf = np.ascontiguousarray(expected_inf, dtype=np.uint8).reshape(6)
+        sg = None if sigmas is None else _u64(sigmas).reshape(3, 4)
+        hr = None if hp_randomness is None else _u64(hp_randomness).reshape(3, 4)
+        out = np.empty((6, 8), dtype=np.uint64)
+        oinf = np.zeros(6, dtype=np.uint8)
+        acc = C.c_int(0)
+        self._check(self._lib.accmsm_nark_as_decide(self._h, C.c_uint64(bases.handle), C.c_uint64(csr), _p(inp), C.c_size_t(inp.shape[0]),
+                                                    _p(wit), C.c_size_t(wit.shape[0]), _p(a), C.c_size_t(a.shape[0]), _p(b),
+                                                    C.c_size_t(b.shape[0]), C.c_size_t(hiding_index), _p(sg), _p(hr), _p(exp), _p(einf),
+                                                    C.byref(acc), _p(out), _p(oinf)), "nark_as_decide")
+        return bool(acc.value), out, oinf
+
     # ---- field-vector kernels
     def compute_coeffs(self, field: int, challenges_mont):
         ch = _u64(challenges_mont).reshape(-1, 4)
@@ -589,8 +609,10 @@ class Bases:
 
 
 from .mirror import (  # noqa: E402
-    ASForHadamardProducts, CommitterKey, InnerProductArgPC, NarkProof, PedersenCommitment, R1CSNark, SuccinctCheckPolynomial, ZkHiding, matrix_vec_mul,
+    AccumulatorInstance, AccumulatorWitness, ASForHadamardProducts, ASForR1CSNark, CommitterKey, InnerProductArgPC, NarkProof, PedersenCommitment,
+    R1CSNark, SuccinctCheckPolynomial, ZkHiding, matrix_vec_mul,
 )
 
 __all__ = ["Context", "Bases", "pinned_array", "release_pinned", "AccmsmError", "PALLAS", "VESTA", "FP", "FQ", "scalar_field", "PedersenCommitment",
-           "CommitterKey", "InnerProductArgPC", "SuccinctCheckPolynomial", "ZkHiding", "ASForHadamardProducts", "R1CSNark", "NarkProof", "matrix_vec_mul"]
+           "CommitterKey", "InnerProductArgPC", "SuccinctCheckPolynomial", "ZkHiding", "ASForHadamardProducts", "R1CSNark", "NarkProof", "ASForR1CSNark",
+           "AccumulatorInstance", "AccumulatorWitness", "matrix_vec_mul"]

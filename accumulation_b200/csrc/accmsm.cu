@@ -982,8 +982,9 @@ int group_register_csr(accmsm_ctx *g, int field, int n_mats, const uint32_t *con
                        const uint64_t *const *coeffs_mont, size_t n_rows, uint64_t *handle);
 int group_release_csr(accmsm_ctx *g, uint64_t handle);
 template <class F>
-int group_csr_pass(accmsm_ctx *g, const std::string &what, uint64_t key_handle, uint64_t csr_handle, size_t n_z, size_t hiding_index,
-                   const uint64_t *tails_mont, size_t m, size_t n_vecs, uint64_t *const *out_vecs, uint64_t *out_xy, uint8_t *out_inf, F run);
+int group_csr_pass(accmsm_ctx *g, const std::string &what, uint64_t key_handle, uint64_t csr_handle, size_t n_z, size_t n_hp,
+                   size_t hiding_index, const uint64_t *tails_mont, size_t m, size_t n_vecs, uint64_t *const *out_vecs, uint64_t *out_xy,
+                   uint8_t *out_inf, F run);
 int group_open_key(accmsm_ctx *g, uint64_t handle, uint64_t *kid0_handle);     // full key on child 0 for IpaPC::open sessions
 // IpaPC::open sessions sharded cyclically across the children of a group (multi_api.inc).  GROUP_IPA_UNSHARDED: the
 // opening is too small to shard / the id is not a sharded session, and child 0 serves the call as before.

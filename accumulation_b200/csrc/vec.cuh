@@ -201,17 +201,23 @@ __global__ void __launch_bounds__(256) k_csr_matvec(CsrMats mats, uint32_t n_row
     store_fe(mats.out[mi] + (size_t)r * 32, acc);
 }
 
-// R1CSNark rows (src/r1cs_nark_as/r1cs_nark/mod.rs:183-261 prove, :335-419 verify): one thread per constraint row walks row r
-// of A, B and C once.  Every (col, coeff) is loaded once and feeds the z-sum over input || witness and, with ZK, the r-sum
-// over 0 || r (input columns add nothing to it).  The products are formed in registers and every result goes straight to
-// row j of the pass's scalar rows (out + j * row_stride):
-//   ZK:  z_A, z_B, z_C, r_A, r_B, r_C, cross = z_A r_B + z_B r_A, rr = r_A r_B
-//   !ZK: t_A, t_B, t_C, t_A t_B
-template <int FIELD, bool ZK>
+// R1CSNark rows (src/r1cs_nark_as/r1cs_nark/mod.rs:183-261 prove, :335-419 verify; the AS decider
+// src/r1cs_nark_as/mod.rs:1031-1112): one thread per constraint row walks row r of A, B and C once.  Every (col, coeff) is
+// loaded once and feeds the z-sum over input || witness and, when proving, the r-sum over 0 || r (input columns add nothing
+// to it).  The products are formed in registers and every result goes straight to row j of the pass's scalar rows
+// (out + j * row_stride):
+//   NARK_PROVE:  z_A, z_B, z_C, r_A, r_B, r_C, cross = z_A r_B + z_B r_A, rr = r_A r_B
+//   NARK_VERIFY: t_A, t_B, t_C, t_A t_B
+//   NARK_DECIDE: t_A, t_B, t_C, a*, b*, a* b*.  The host has uploaded a*[0, n_a) into row 3 and b*[0, n_b) into row 4; the
+//                thread reads its entry there (zero at or beyond the length, and stores that zero), so every scalar of the
+//                six rows is written before the pass reads it.
+enum NarkMode : int { NARK_PROVE, NARK_VERIFY, NARK_DECIDE };
+template <int FIELD, int MODE>
 __global__ void __launch_bounds__(256) k_nark_rows(CsrMats mats, uint32_t n_rows, const uint8_t *__restrict__ input, uint32_t n_input,
                                                     const uint8_t *__restrict__ witness, const uint8_t *__restrict__ rvec,
-                                                    uint8_t *__restrict__ out, size_t row_stride) {
+                                                    uint8_t *__restrict__ out, size_t row_stride, uint32_t n_a, uint32_t n_b) {
     using F = Fp<FIELD>;
+    constexpr bool ZK = MODE == NARK_PROVE;
     uint32_t r = blockIdx.x * blockDim.x + threadIdx.x;
     if (r >= n_rows) return;
     const fe_t one = F::one();
@@ -245,8 +251,14 @@ __global__ void __launch_bounds__(256) k_nark_rows(CsrMats mats, uint32_t n_rows
     if (ZK) {
         store_fe(out + (size_t)6 * row_stride + (size_t)r * 32, F::add(F::mul(za, rb), F::mul(zb, ra)));
         store_fe(out + (size_t)7 * row_stride + (size_t)r * 32, F::mul(ra, rb));
-    } else {
+    } else if (MODE == NARK_VERIFY) {
         store_fe(out + (size_t)3 * row_stride + (size_t)r * 32, F::mul(za, zb));
+    } else {
+        uint8_t *pa = out + (size_t)3 * row_stride + (size_t)r * 32, *pb = out + (size_t)4 * row_stride + (size_t)r * 32;
+        fe_t a = F::zero(), b = F::zero();
+        if (r < n_a) a = load_fe(pa); else store_fe(pa, a);
+        if (r < n_b) b = load_fe(pb); else store_fe(pb, b);
+        store_fe(out + (size_t)5 * row_stride + (size_t)r * 32, F::mul(a, b));
     }
 }
 

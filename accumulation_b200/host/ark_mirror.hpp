@@ -13,6 +13,8 @@
 //   r1cs_nark: Matrix<F> = Vec<Vec<(F, usize)>>, matrix_vec_mul,       r1cs_nark::{Matrix, matrix_vec_mul, IndexMatrices}
 //              R1CSNark::prove (zk first message) / verify             IndexMatrices::{matvec_commit, prove_zk, verify}
 //                                        (src/r1cs_nark_as/r1cs_nark/mod.rs:183-419, 443-462)
+//   r1cs_nark_as: AccumulatorInstance, AccumulatorWitness, decide       r1cs_nark_as::{AccumulatorInstance, AccumulatorWitness, decide}
+//                                        (src/r1cs_nark_as/data_structures.rs:156-227, src/r1cs_nark_as/mod.rs:1031-1112)
 // Every call computes on the GPU; there is no CPU path.  ark's commit is infallible -> failures throw AccmsmError
 // (the Rust wrapper panics / maps to PCError at the same places).
 #pragma once
@@ -376,7 +378,10 @@ inline std::vector<std::vector<Fe>> matrix_vec_mul(const Context &ctx, int field
 // IndexProverKey{a, b, c, ck} with the matrices resident on the device (registered at index time)
 class IndexMatrices {
 public:
-    IndexMatrices(const CommitterKey &ck, const Matrix &a, const Matrix &b, const Matrix &c) : ck_(ck), n_rows_(a.size()) {
+    // num_instance_variables: the index's input length (IndexInfo), which r1cs_nark_as::decide checks r1cs_input against
+    IndexMatrices(const CommitterKey &ck, const Matrix &a, const Matrix &b, const Matrix &c,
+                  std::optional<size_t> num_instance_variables = std::nullopt)
+        : ck_(ck), n_rows_(a.size()), num_instance_variables_(num_instance_variables) {
         Csr ca = to_csr(a), cb = to_csr(b), cc = to_csr(c);
         const uint32_t *rp[3] = {ca.row_ptr.data(), cb.row_ptr.data(), cc.row_ptr.data()};
         const uint32_t *cl[3] = {ca.cols.data(), cb.cols.data(), cc.cols.data()};
@@ -385,6 +390,8 @@ public:
     }
     ~IndexMatrices() { accmsm_release_csr(ck_.ctx()->raw(), handle_); }
     uint64_t handle() const { return handle_; }
+    const CommitterKey &ck() const { return ck_; }
+    std::optional<size_t> num_instance_variables() const { return num_instance_variables_; }
     // z_M = M (input || witness), comm_M = Commit(z_M, blinder_M)   (prove :183-185 + :216-218; decide src/r1cs_nark_as/mod.rs:1052-1097)
     std::pair<std::vector<std::vector<Fe>>, std::vector<Affine>> matvec_commit(const std::vector<Fe> &input, const std::vector<Fe> &witness,
                                                                               const std::optional<std::array<Fe, 3>> &blinders = std::nullopt) const {
@@ -437,8 +444,54 @@ public:
 private:
     const CommitterKey &ck_;
     size_t n_rows_;
+    std::optional<size_t> num_instance_variables_;
     uint64_t handle_ = 0;
 };
 }  // namespace r1cs_nark
+
+namespace r1cs_nark_as {
+// src/r1cs_nark_as/data_structures.rs:156-171, :218-227
+struct AccumulatorInstance {
+    std::vector<Fe> r1cs_input;
+    Affine comm_a, comm_b, comm_c;
+    ASForHadamardProducts::InputInstance hp_instance;
+};
+struct AccumulatorWitnessRandomness { Fe sigma_a, sigma_b, sigma_c; };
+struct AccumulatorWitness {
+    std::vector<Fe> r1cs_blinded_witness;
+    ASForHadamardProducts::InputWitness hp_witness;
+    std::optional<AccumulatorWitnessRandomness> randomness;
+};
+// ASForR1CSNark::decide (src/r1cs_nark_as/mod.rs:1031-1112): t_M = M (r1cs_input || r1cs_blinded_witness); accept iff
+// Commit(t_M, sigma_M) == comm_M for M = A, B, C and hp_as::decide(ck, hp_instance, hp_witness), in ONE library call (one
+// vector launch, the six commitments in one pass).  An r1cs_input whose length differs from the index's is rejected here.
+inline bool decide(const r1cs_nark::IndexMatrices &index, const AccumulatorInstance &instance, const AccumulatorWitness &witness) {
+    const CommitterKey &ck = index.ck();
+    if (index.num_instance_variables() && instance.r1cs_input.size() != *index.num_instance_variables()) return false;
+    const auto &hw = witness.hp_witness;
+    if ((witness.randomness || hw.randomness) && !ck.has_hiding()) throw AccmsmError("decide: the key has no hiding generator");
+    const Affine *pts[6] = {&instance.comm_a, &instance.comm_b, &instance.comm_c, &instance.hp_instance.comm_1,
+                            &instance.hp_instance.comm_2, &instance.hp_instance.comm_3};
+    uint64_t exp[48]; uint8_t einf[6];
+    for (int j = 0; j < 6; j++) { affine_to(*pts[j], exp + 8 * j); einf[j] = pts[j]->infinity; }
+    uint64_t sig[12], hr[12];
+    if (witness.randomness) {
+        std::memcpy(sig, witness.randomness->sigma_a.data(), 32); std::memcpy(sig + 4, witness.randomness->sigma_b.data(), 32);
+        std::memcpy(sig + 8, witness.randomness->sigma_c.data(), 32);
+    }
+    if (hw.randomness) {
+        std::memcpy(hr, hw.randomness->rand_1.data(), 32); std::memcpy(hr + 4, hw.randomness->rand_2.data(), 32);
+        std::memcpy(hr + 8, hw.randomness->rand_3.data(), 32);
+    }
+    const auto &x = instance.r1cs_input, &w = witness.r1cs_blinded_witness;
+    int accept = 0;
+    ck.ctx()->check(accmsm_nark_as_decide(ck.ctx()->raw(), ck.handle(), index.handle(), x.empty() ? nullptr : x[0].data(), x.size(),
+                                          w.empty() ? nullptr : w[0].data(), w.size(), hw.a_vec.empty() ? nullptr : hw.a_vec[0].data(),
+                                          hw.a_vec.size(), hw.b_vec.empty() ? nullptr : hw.b_vec[0].data(), hw.b_vec.size(),
+                                          ck.hiding_index(), witness.randomness ? sig : nullptr, hw.randomness ? hr : nullptr, exp, einf,
+                                          &accept, nullptr, nullptr), "nark_as_decide");
+    return accept != 0;
+}
+}  // namespace r1cs_nark_as
 
 }  // namespace accmsm_host

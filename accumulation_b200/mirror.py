@@ -327,9 +327,11 @@ class R1CSNark:
     """The mat-vec + commitment steps of src/r1cs_nark_as/r1cs_nark/mod.rs (prove :183-316, verify :335-419) and of
     ASForR1CSNark::decide (src/r1cs_nark_as/mod.rs:1052-1097) with the index matrices registered once."""
 
-    def __init__(self, ck: CommitterKey, matrices):
+    def __init__(self, ck: CommitterKey, matrices, num_instance_variables: Optional[int] = None):
+        """num_instance_variables: the index's input length (IndexInfo), which ASForR1CSNark.decide checks r1cs_input against"""
         from . import scalar_field
         self.ck = ck
+        self.num_instance_variables = num_instance_variables
         self.n_mats = len(matrices)
         self.n_rows = int(np.asarray(matrices[0][0]).size - 1)
         self.csr = ck.bases.ctx.register_csr(scalar_field(ck.curve), matrices)
@@ -386,3 +388,46 @@ class R1CSNark:
 
     def release(self):
         self.ck.bases.ctx.release_csr(self.csr)
+
+
+@dataclass
+class AccumulatorInstance:
+    """r1cs_nark_as::AccumulatorInstance (src/r1cs_nark_as/data_structures.rs:156-171): comm_a, comm_b, comm_c and the
+    hp_instance (comm_1, comm_2, comm_3) as (xy, inf)."""
+    r1cs_input: "object"
+    comm_a: tuple
+    comm_b: tuple
+    comm_c: tuple
+    hp_instance: tuple
+
+
+@dataclass
+class AccumulatorWitness:
+    """r1cs_nark_as::AccumulatorWitness (src/r1cs_nark_as/data_structures.rs:218-227): hp_witness = (a_vec, b_vec,
+    randomness | None) as in ASForHadamardProducts.decide; randomness = (sigma_a, sigma_b, sigma_c) or None."""
+    r1cs_blinded_witness: "object"
+    hp_witness: tuple
+    randomness: "object" = None
+
+
+class ASForR1CSNark:
+    """The decider of src/r1cs_nark_as/mod.rs (:1031-1112) over an R1CSNark index (matrices registered once)."""
+
+    @staticmethod
+    def decide(nark: R1CSNark, instance: AccumulatorInstance, witness: AccumulatorWitness) -> bool:
+        """t_M = M (r1cs_input || r1cs_blinded_witness); accept iff Commit(t_M, sigma_M) == comm_M for M = A, B, C and the hp
+        decider accepts (a*, b*, randomness) against hp_instance.  One nark_as_decide call: one vector launch, the six
+        commitments in one 6-job pass, the comparison.  An r1cs_input whose length differs from the index's is rejected on
+        the host."""
+        x = np.ascontiguousarray(instance.r1cs_input, dtype=np.uint64).reshape(-1, 4)
+        if nark.num_instance_variables is not None and x.shape[0] != nark.num_instance_variables:
+            return False
+        a_vec, b_vec, hp_rand = witness.hp_witness
+        pts = [instance.comm_a, instance.comm_b, instance.comm_c, *instance.hp_instance]
+        exp_xy = np.array([np.asarray(p[0], dtype=np.uint64) for p in pts])
+        exp_inf = np.array([int(p[1]) for p in pts], dtype=np.uint8)
+        sig = None if witness.randomness is None else np.array([np.asarray(v, dtype=np.uint64) for v in witness.randomness])
+        hr = None if hp_rand is None else np.array([np.asarray(v, dtype=np.uint64) for v in hp_rand])
+        ok, _, _ = nark.ck.bases.ctx.nark_as_decide(nark.ck.bases, nark.csr, x, witness.r1cs_blinded_witness, a_vec, b_vec, exp_xy, exp_inf,
+                                                     hiding_index=nark.ck.num_generators, sigmas=sig, hp_randomness=hr)
+        return ok

@@ -363,6 +363,17 @@ int accmsm_nark_verify(accmsm_ctx *ctx, uint64_t key_handle, uint64_t csr_handle
                        const uint64_t *blinded_witness, size_t n_witness, size_t hiding_index, const uint64_t *sigmas_mont,
                        const uint64_t *expected_xy, const uint8_t *expected_inf, int *accept, uint64_t *out_xy,
                        uint8_t *out_inf, uint64_t *const *out_vecs);
+/* ASForR1CSNark::decide (src/r1cs_nark_as/mod.rs:1031-1112): t_M = M (x*||w*) for the 3 matrices of csr_handle, then
+ * Commit(t_M, sigma_M*) for M = A, B, C, and the hp decider's Commit(a*, r1*), Commit(b*, r2*), Commit(a* o b*, r3*)
+ * (src/hp_as/mod.rs:894-925), all six in ONE pass; accept iff they equal expected_xy / expected_inf in the order
+ * comm_A*, comm_B*, comm_C*, C1*, C2*, C3* (out_xy / out_inf, nullable, in the same order).
+ * hp_a, hp_b: a* and b* with n_a, n_b <= n_rows (else ACCMSM_E_ARG); the product runs over min(n_a, n_b).
+ * sigmas: (sigma_A*, sigma_B*, sigma_C*), hp_rand: (r1*, r2*, r3*), each 3 x 4 or NULL; an absent triple adds nothing.
+ * One pass of 6 jobs over n_rows + 1 pairs needs 6 x windows x (n_rows + 1) < 2^31: n_rows <= 27,531,840 (~2^24.7) at c = 20. */
+int accmsm_nark_as_decide(accmsm_ctx *ctx, uint64_t key_handle, uint64_t csr_handle, const uint64_t *input, size_t n_input,
+                          const uint64_t *witness, size_t n_witness, const uint64_t *hp_a, size_t n_a, const uint64_t *hp_b, size_t n_b,
+                          size_t hiding_index, const uint64_t *sigmas_mont, const uint64_t *hp_rand_mont, const uint64_t *expected_xy,
+                          const uint8_t *expected_inf, int *accept, uint64_t *out_xy, uint8_t *out_inf);
 
 #ifdef __cplusplus
 }
