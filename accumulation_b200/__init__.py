@@ -501,6 +501,49 @@ class Context:
                                                     C.byref(acc), _p(out), _p(oinf)), "nark_as_decide")
         return bool(acc.value), out, oinf
 
+    def hp_prove_begin(self, bases: "Bases", a_vecs, b_vecs, length: int, hiding_a=None, hiding_b=None, hiding_index: int = 0,
+                       hiding_rand=None):
+        """ASForHadamardProducts::prove, first step: the n pairs (a_i, b_i) go to HBM once and stay there until
+        hp_prove_finish.  With hiding (ha, hb of `length` elements, hiding_rand = (r1, r2, r3)) the three hiding commitments
+        Commit(ha, r1), Commit(hb, r2), Commit(ha o b_0 + a_{n-1} o hb, r3) come from one pass -> (session, (xy (3, 8),
+        inf (3,)) | None)"""
+        a_vecs = [_u64(v).reshape(-1, 4) for v in a_vecs]
+        b_vecs = [_u64(v).reshape(-1, 4) for v in b_vecs]
+        n = len(a_vecs)
+        al = np.array([v.shape[0] for v in a_vecs], dtype=np.uint64)
+        bl = np.array([v.shape[0] for v in b_vecs], dtype=np.uint64)
+        ha = None if hiding_a is None else _u64(hiding_a).reshape(-1, 4)
+        hb = None if hiding_b is None else _u64(hiding_b).reshape(-1, 4)
+        hr = None if hiding_rand is None else _u64(hiding_rand).reshape(3, 4)
+        out, oinf = np.zeros((3, 8), dtype=np.uint64), np.zeros(3, dtype=np.uint8)
+        sess = C.c_uint64(0)
+        self._check(self._lib.accmsm_hp_prove_begin(self._h, C.c_uint64(bases.handle), self._ptrs(a_vecs), _p(al), self._ptrs(b_vecs),
+                                                    _p(bl), C.c_int(n), C.c_size_t(length), _p(ha), _p(hb), C.c_size_t(hiding_index),
+                                                    _p(hr), _p(out), _p(oinf), C.byref(sess)), "hp_prove_begin")
+        return int(sess.value), (None if ha is None else (out, oinf))
+
+    def hp_prove_product_poly_comm(self, session: int, n: int, mu):
+        """second step: t-vectors of the resident pairs and their 2n - 2 commitments; mu has n entries (n + 1 with hiding:
+        mu_n = mu_1 mu_{n-1}) -> ((low xy (n-1, 8), inf), (high xy (n-1, 8), inf))"""
+        mu = _u64(mu).reshape(-1, 4)
+        low, high = np.empty((max(n - 1, 0), 8), dtype=np.uint64), np.empty((max(n - 1, 0), 8), dtype=np.uint64)
+        linf, hinf = np.zeros(max(n - 1, 0), dtype=np.uint8), np.zeros(max(n - 1, 0), dtype=np.uint8)
+        self._check(self._lib.accmsm_hp_prove_product_poly_comm(self._h, C.c_uint64(session), _p(mu), C.c_size_t(mu.shape[0]), _p(low),
+                                                                _p(linf), _p(high), _p(hinf)), "hp_prove_product_poly_comm")
+        return (low, linf), (high, hinf)
+
+    def hp_prove_finish(self, session: int, nu, capacity: int):
+        """last step: a* = mu_n ha + sum_i mu_i nu^i a_i, b* = mu_1 hb + sum_j nu^j b_{n-1-j}; releases the session (on error
+        too) -> (a*, b*)"""
+        a, b = np.empty((capacity, 4), dtype=np.uint64), np.empty((capacity, 4), dtype=np.uint64)
+        olen = (C.c_size_t * 2)()
+        self._check(self._lib.accmsm_hp_prove_finish(self._h, C.c_uint64(session), _p(_u64(nu)), _p(a), _p(b), C.c_size_t(capacity), olen),
+                    "hp_prove_finish")
+        return a[: olen[0]], b[: olen[1]]
+
+    def hp_prove_abort(self, session: int):
+        self._check(self._lib.accmsm_hp_prove_abort(self._h, C.c_uint64(session)), "hp_prove_abort")
+
     # ---- field-vector kernels
     def compute_coeffs(self, field: int, challenges_mont):
         ch = _u64(challenges_mont).reshape(-1, 4)

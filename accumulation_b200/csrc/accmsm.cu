@@ -8,6 +8,7 @@
 #include <cstdlib>
 #include <cstring>
 #include <functional>
+#include <memory>
 #include <mutex>
 #include <string>
 #include <unordered_map>
@@ -60,6 +61,8 @@ struct IpaSession;
 void ipa_session_free(IpaSession *s);
 struct CsrSet;
 void csr_set_free(CsrSet *c);
+struct HpSession;
+void hp_session_free(accmsm_ctx *ctx, HpSession *s);
 
 struct GroupWorker;
 struct GroupKey;
@@ -73,6 +76,7 @@ struct accmsm_ctx {
     std::unordered_map<uint64_t, GroupKey *> gkeys;
     std::unordered_map<uint64_t, GroupCsr *> gcsrs;
     std::unordered_map<uint64_t, struct GroupIpaSession *> gsessions;   // IpaPC::open sessions sharded across the children
+    std::unordered_map<uint64_t, struct GroupHpSession *> ghp_sessions; // hp-as prover sessions over the children's columns
     std::vector<char> peer_ok;                           // child g can store straight into child 0's memory
     std::vector<char> peer_read;                         // [i * children + j]: child i's kernels can read child j's memory
     void *d_gather = nullptr;                            // on child 0's device: partial sums of all children, rank-major
@@ -86,6 +90,7 @@ struct accmsm_ctx {
     std::unordered_map<uint64_t, struct IpaSession *> ipa_sessions;
     std::vector<struct IpaSession *> ipa_free;
     std::unordered_map<uint64_t, struct CsrSet *> csr_sets;
+    std::unordered_map<uint64_t, HpSession *> hp_sessions;  // ASForHadamardProducts::prove sessions (fused_api.inc)
     std::vector<std::pair<void *, size_t>> vec_cache;   // recycled scratch blocks of the field-vector entry points
     uint64_t next_handle = 1;
     int window_bits = 0;
@@ -986,6 +991,16 @@ int group_csr_pass(accmsm_ctx *g, const std::string &what, uint64_t key_handle, 
                    size_t hiding_index, const uint64_t *tails_mont, size_t m, size_t n_vecs, uint64_t *const *out_vecs, uint64_t *out_xy,
                    uint8_t *out_inf, F run);
 int group_open_key(accmsm_ctx *g, uint64_t handle, uint64_t *kid0_handle);     // full key on child 0 for IpaPC::open sessions
+// hp-as prover sessions: every child holds the columns of its key shard
+int group_hp_prove_begin(accmsm_ctx *g, uint64_t key_handle, const uint64_t *const *a_vecs, const size_t *a_lens,
+                         const uint64_t *const *b_vecs, const size_t *b_lens, int n, size_t len, const uint64_t *hiding_a,
+                         const uint64_t *hiding_b, size_t hiding_index, const uint64_t *rand_mont, uint64_t *comm_xy, uint8_t *comm_inf,
+                         uint64_t *session);
+int group_hp_prove_ppc(accmsm_ctx *g, uint64_t session, const uint64_t *mu_mont, size_t n_mu, uint64_t *low_xy, uint8_t *low_inf,
+                       uint64_t *high_xy, uint8_t *high_inf);
+int group_hp_prove_finish(accmsm_ctx *g, uint64_t session, const uint64_t nu_mont[4], uint64_t *a_star, uint64_t *b_star, size_t capacity,
+                          size_t *out_len);
+int group_hp_prove_abort(accmsm_ctx *g, uint64_t session);
 // IpaPC::open sessions sharded cyclically across the children of a group (multi_api.inc).  GROUP_IPA_UNSHARDED: the
 // opening is too small to shard / the id is not a sharded session, and child 0 serves the call as before.
 constexpr int GROUP_IPA_UNSHARDED = 1;
@@ -1111,6 +1126,7 @@ void accmsm_destroy(accmsm_ctx *ctx) {
     for (auto &kv : ctx->ipa_sessions) ipa_session_free(kv.second);
     for (auto *fs : ctx->ipa_free) ipa_session_free(fs);
     for (auto &kv : ctx->csr_sets) csr_set_free(kv.second);
+    for (auto &kv : ctx->hp_sessions) hp_session_free(ctx, kv.second);     // before the cache their blocks return to
     for (auto &b : ctx->vec_cache) cudaFree(b.first);
     ctx->digits.release(); ctx->hist.release(); ctx->offsets.release(); ctx->cursor.release(); ctx->entries.release();
     ctx->cta_ids.release(); ctx->tile_sums.release(); ctx->tile_offs.release(); ctx->buckets.release(); ctx->cta_parts.release(); ctx->partial.release();

@@ -129,15 +129,20 @@ __global__ void __launch_bounds__(256) k_scale(const uint8_t *__restrict__ v, ui
     if (i >= n) return;
     store_fe(out + (size_t)i * 32, Fp<FIELD>::mul(load_fe_nc(v + (size_t)i * 32), load_fe(c)));
 }
-// out[li] = hiding[li] + sum_ni ch[ni] * vecs[ni][li]   (ragged inputs: missing elements are skipped)
+// out[li] = h * hiding[li] + sum_ni ch[ni] * vecs[ni][li]   (ragged inputs: missing elements are skipped; h = *hiding_ch, or 1
+// when hiding_ch is null)
 template <int FIELD>
 __global__ void __launch_bounds__(256) k_lincomb(VecPtrs vecs, int m, const uint8_t *__restrict__ ch,
                                                   const uint8_t *__restrict__ hiding, uint32_t n_hiding, uint32_t out_len,
-                                                  uint8_t *__restrict__ out) {
+                                                  uint8_t *__restrict__ out, const uint8_t *__restrict__ hiding_ch) {
     using F = Fp<FIELD>;
     uint32_t li = blockIdx.x * blockDim.x + threadIdx.x;
     if (li >= out_len) return;
-    fe_t acc = (hiding && li < n_hiding) ? load_fe_nc(hiding + (size_t)li * 32) : F::zero();
+    fe_t acc = F::zero();
+    if (hiding && li < n_hiding) {
+        acc = load_fe_nc(hiding + (size_t)li * 32);
+        if (hiding_ch) acc = F::mul(acc, load_fe(hiding_ch));
+    }
     for (int ni = 0; ni < m; ni++) {
         if (li < vecs.len[ni]) acc = F::add(acc, F::mul(load_fe(ch + (size_t)ni * 32), load_fe_nc(vecs.ptr[ni] + (size_t)li * 32)));
     }
@@ -173,6 +178,28 @@ __global__ void __launch_bounds__(TVEC_THREADS) k_tvecs(VecPtrs a, VecPtrs b, in
         for (int i = i0; i <= i1; i++) acc = F::add(acc, F::mul(A[i * TVEC_THREADS + threadIdx.x], Bp[(k - i) * TVEC_THREADS + threadIdx.x]));
         store_fe(out + ((size_t)k * len + li) * 32, acc);
     }
+}
+
+// zk hiding rows of ASForHadamardProducts::prove (src/hp_as/mod.rs:179-230), straight into the first three rows of a pass's
+// scalar buffer (out + j * row_stride): ha, hb, and cross = ha o b_0 + a_{n-1} o hb, the hiding part of the middle t-vector
+// (SURVEY.md App. C.3: T[n-1] carries mu_n (ha o b_0 + a_{n-1} o hb) for n >= 2).  b_0 and a_{n-1} are ragged (zero beyond their
+// lengths); ha and hb have len elements.
+template <int FIELD>
+__global__ void __launch_bounds__(256) k_hp_hiding_rows(const uint8_t *__restrict__ ha, const uint8_t *__restrict__ hb,
+                                                         const uint8_t *__restrict__ b_first, uint32_t n_b_first,
+                                                         const uint8_t *__restrict__ a_last, uint32_t n_a_last, uint32_t len,
+                                                         uint8_t *__restrict__ out, size_t row_stride) {
+    using F = Fp<FIELD>;
+    uint32_t li = blockIdx.x * blockDim.x + threadIdx.x;
+    if (li >= len) return;
+    const size_t o = (size_t)li * 32;
+    const fe_t h_a = load_fe_nc(ha + o), h_b = load_fe_nc(hb + o);
+    fe_t cross = F::zero();
+    if (li < n_b_first) cross = F::mul(h_a, load_fe_nc(b_first + o));
+    if (li < n_a_last) cross = F::add(cross, F::mul(load_fe_nc(a_last + o), h_b));
+    store_fe(out + o, h_a);
+    store_fe(out + row_stride + o, h_b);
+    store_fe(out + 2 * row_stride + o, cross);
 }
 
 // CSR sparse mat-vec, up to 3 matrices over the same z = input || witness; one thread per (matrix, row)

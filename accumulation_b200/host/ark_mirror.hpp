@@ -9,7 +9,7 @@
 //   ipa_pc::InnerProductArgPC::cm_commit / check (final key) / open    InnerProductArgPC::{cm_commit, check_final_key, open}
 //   ipa_pc::SuccinctCheckPolynomial(Vec<F>)::compute_coeffs            SuccinctCheckPolynomial::compute_coeffs
 //   hp_as: compute_hp, compute_t_vecs, combine_vectors, scale_vector,  ASForHadamardProducts::...
-//          compute_product_poly_comm, decide   (src/hp_as/mod.rs:278-512, 894-925)
+//          compute_product_poly_comm, prove, verify, decide   (src/hp_as/mod.rs:278-512, 646-925)
 //   r1cs_nark: Matrix<F> = Vec<Vec<(F, usize)>>, matrix_vec_mul,       r1cs_nark::{Matrix, matrix_vec_mul, IndexMatrices}
 //              R1CSNark::prove (zk first message) / verify             IndexMatrices::{matvec_commit, prove_zk, verify}
 //                                        (src/r1cs_nark_as/r1cs_nark/mod.rs:183-419, 443-462)
@@ -30,6 +30,7 @@
 #include <vector>
 
 #include "../../include/accmsm.h"
+#include "../csrc/hostfp.hpp"
 
 namespace accmsm_host {
 
@@ -347,6 +348,133 @@ struct ASForHadamardProducts {
         ck.ctx()->check(accmsm_hp_decide(ck.ctx()->raw(), ck.handle(), n ? witness.a_vec[0].data() : nullptr, n ? witness.b_vec[0].data() : nullptr, n,
                                          ck.hiding_index(), witness.randomness ? r : nullptr, exp, einf, &accept, nullptr, nullptr), "hp_decide");
         return accept != 0;
+    }
+
+    // prove (:646-813) over the already padded pairs, inputs first, then old accumulators (the placeholder padding of :676-710
+    // stays with the caller).  The sponge is the callables: mu_of(hiding_comms) -> mu_1 .. mu_{n-1}, nu_of(low, high) -> nu.
+    // One device session (accmsm_hp_prove_*) forms the hiding commitments, the product-polynomial commitments and a*, b*; the
+    // randomness (App. C.5) is host arithmetic and the new instance (C.6) one 3-equation batched MSM, as upstream.
+    struct Proof { std::optional<std::array<Affine, 3>> hiding_comms; std::vector<Affine> low, high; };   // src/hp_as/data_structures.rs
+    struct HidingVecs { std::vector<Fe> a_vec, b_vec; Randomness randomness; };                           // hp_vec_len elements each
+    using MuOf = std::function<std::vector<Fe>(const std::optional<std::array<Affine, 3>> &)>;
+    using NuOf = std::function<Fe(const std::vector<Affine> &, const std::vector<Affine> &)>;
+    struct ProveOutput { InputInstance instance; InputWitness witness; Proof proof; };
+    static ProveOutput prove(const CommitterKey &ck, const std::vector<InputWitness> &witnesses, const std::vector<InputInstance> &instances,
+                             const MuOf &mu_of, const NuOf &nu_of, const std::optional<HidingVecs> &zk = std::nullopt) {
+        const size_t n = witnesses.size(), L = ck.supported_num_elems();
+        const accmsm::hostfp::Modulus &M = accmsm::hostfp::modulus(scalar_field(ck.curve()));
+        if (zk && !ck.has_hiding()) throw AccmsmError("prove: the key has no hiding generator");
+        if (instances.size() != n) throw AccmsmError("prove: one instance per witness");
+        std::vector<const uint64_t *> ap, bp; std::vector<size_t> al, bl;
+        for (const auto &w : witnesses) {
+            al.push_back(std::min(w.a_vec.size(), L)); ap.push_back(al.back() ? w.a_vec[0].data() : nullptr);
+            bl.push_back(std::min(w.b_vec.size(), L)); bp.push_back(bl.back() ? w.b_vec[0].data() : nullptr);
+        }
+        accmsm_ctx *c = ck.ctx()->raw();
+        uint64_t hr[12], hxy[24], sess = 0; uint8_t hinf[3] = {0, 0, 0};
+        std::vector<Fe> ha, hb;
+        if (zk) {
+            ha = zk->a_vec; hb = zk->b_vec;
+            ha.resize(L); hb.resize(L);        // hp_vec_len elements (zero padded)
+            std::memcpy(hr, zk->randomness.rand_1.data(), 32); std::memcpy(hr + 4, zk->randomness.rand_2.data(), 32);
+            std::memcpy(hr + 8, zk->randomness.rand_3.data(), 32);
+        }
+        const std::vector<Fe> zero(1);
+        ck.ctx()->check(accmsm_hp_prove_begin(c, ck.handle(), ap.data(), al.data(), bp.data(), bl.data(), (int)n, L,
+                                              zk ? (L ? ha[0].data() : zero[0].data()) : nullptr, zk ? (L ? hb[0].data() : zero[0].data()) : nullptr,
+                                              ck.hiding_index(), zk ? hr : nullptr, hxy, hinf, &sess), "hp_prove_begin");
+        ProveOutput out;
+        std::vector<Fe> mu(1, Fe{M.one[0], M.one[1], M.one[2], M.one[3]});
+        try {
+            if (zk) out.proof.hiding_comms = std::array<Affine, 3>{affine_from(hxy, hinf[0]), affine_from(hxy + 8, hinf[1]), affine_from(hxy + 16, hinf[2])};
+            const std::vector<Fe> mus = mu_of(out.proof.hiding_comms);
+            if (mus.size() + 1 != n) throw AccmsmError("prove: mu_of must return n - 1 challenges");
+            mu.insert(mu.end(), mus.begin(), mus.end());
+            if (zk) { Fe mn; accmsm::hostfp::mul(M, mu[1].data(), mu[n - 1].data(), mn.data()); mu.push_back(mn); }
+            std::vector<uint64_t> lo(8 * n), hi(8 * n); std::vector<uint8_t> li(n), hinf2(n);
+            ck.ctx()->check(accmsm_hp_prove_product_poly_comm(c, sess, mu[0].data(), mu.size(), lo.data(), li.data(), hi.data(), hinf2.data()),
+                            "hp_prove_product_poly_comm");
+            for (size_t j = 0; j + 1 < n; j++) { out.proof.low.push_back(affine_from(&lo[8 * j], li[j])); out.proof.high.push_back(affine_from(&hi[8 * j], hinf2[j])); }
+        } catch (...) {
+            accmsm_hp_prove_abort(c, sess);
+            throw;
+        }
+        const Fe nu = nu_of(out.proof.low, out.proof.high);
+        std::vector<Fe> a_star(L), b_star(L);
+        size_t olen[2] = {0, 0};
+        ck.ctx()->check(accmsm_hp_prove_finish(c, sess, nu.data(), L ? a_star[0].data() : nullptr, L ? b_star[0].data() : nullptr, L, olen),
+                        "hp_prove_finish");
+        a_star.resize(olen[0]); b_star.resize(olen[1]);
+        out.witness.a_vec = std::move(a_star); out.witness.b_vec = std::move(b_star);
+        const std::vector<Fe> nus = powers(M, nu, 2 * n - 1);
+        if (zk) {       // App. C.5; absent randomness entries add nothing
+            Fe r1 = mul(M, mu[n], zk->randomness.rand_1), r2 = mul(M, mu[1], zk->randomness.rand_2), r3 = mul(M, mu[n], zk->randomness.rand_3);
+            for (size_t i = 0; i < n; i++) {
+                if (const auto &r = witnesses[i].randomness) {
+                    r1 = add(M, r1, mul(M, mul(M, mu[i], nus[i]), r->rand_1));
+                    r3 = add(M, r3, mul(M, mu[i], r->rand_3));
+                }
+                if (const auto &r = witnesses[n - 1 - i].randomness) r2 = add(M, r2, mul(M, nus[i], r->rand_2));
+            }
+            out.witness.randomness = Randomness{r1, r2, mul(M, r3, nus[n - 1])};
+        }
+        out.instance = combined_commitments(ck, instances, out.proof, mu, nu);
+        return out;
+    }
+    // verify (:815-892): mu and nu from the same sponge, C1*, C2*, C3* recomputed from the old instances and the proof; accept iff
+    // they equal new_instance.  A proof whose shape does not fit n is rejected.
+    static bool verify(const CommitterKey &ck, const std::vector<InputInstance> &instances, const InputInstance &new_instance, const Proof &proof,
+                       const MuOf &mu_of, const NuOf &nu_of) {
+        const size_t n = instances.size();
+        const accmsm::hostfp::Modulus &M = accmsm::hostfp::modulus(scalar_field(ck.curve()));
+        if (n < 1 || proof.low.size() != n - 1 || proof.high.size() != n - 1) return false;
+        std::vector<Fe> mu(1, Fe{M.one[0], M.one[1], M.one[2], M.one[3]});
+        const std::vector<Fe> mus = mu_of(proof.hiding_comms);
+        if (mus.size() + 1 != n) return false;
+        mu.insert(mu.end(), mus.begin(), mus.end());
+        if (proof.hiding_comms) { if (n < 2) return false; mu.push_back(mul(M, mu[1], mu[n - 1])); }
+        const InputInstance got = combined_commitments(ck, instances, proof, mu, nu_of(proof.low, proof.high));
+        return got.comm_1 == new_instance.comm_1 && got.comm_2 == new_instance.comm_2 && got.comm_3 == new_instance.comm_3;
+    }
+    // compute_combined_hp_commitments (:409-479, App. C.6): C1* = [mu_n H1] + sum_i mu_i nu^i C1_i, C2* = [mu_1 H2] + sum_j nu^j C2_{n-1-j},
+    // C3* = sum_j nu^j low_j + sum_j nu^(n+j) high_j + nu^(n-1) ([mu_n H3] + sum_i mu_i C3_i), one batched MSM of 3 equations
+    static InputInstance combined_commitments(const CommitterKey &ck, const std::vector<InputInstance> &instances, const Proof &proof,
+                                              const std::vector<Fe> &mu, const Fe &nu) {
+        const size_t n = instances.size();
+        const accmsm::hostfp::Modulus &M = accmsm::hostfp::modulus(scalar_field(ck.curve()));
+        const std::vector<Fe> nus = powers(M, nu, 2 * n - 1);
+        std::vector<std::vector<Affine>> pts(3);
+        std::vector<std::vector<Fe>> sc(3);
+        auto term = [&](int e, const Affine &p, const Fe &s) { pts[e].push_back(p); sc[e].push_back(canonical(M, s)); };
+        for (size_t i = 0; i < n; i++) {
+            term(0, instances[i].comm_1, mul(M, mu[i], nus[i]));
+            term(1, instances[n - 1 - i].comm_2, nus[i]);
+            term(2, instances[i].comm_3, mul(M, mu[i], nus[n - 1]));
+        }
+        for (size_t j = 0; j + 1 < n; j++) { term(2, proof.low[j], nus[j]); term(2, proof.high[j], nus[n + j]); }
+        if (proof.hiding_comms) {
+            term(0, (*proof.hiding_comms)[0], mu[n]);
+            term(1, (*proof.hiding_comms)[1], mu[1]);
+            term(2, (*proof.hiding_comms)[2], mul(M, mu[n], nus[n - 1]));
+        }
+        size_t width = 0;
+        for (const auto &e : pts) width = std::max(width, e.size());
+        for (int e = 0; e < 3; e++) while (pts[e].size() < width) {     // (a point flagged as the identity, 0)
+            Affine p = pts[e][0]; p.infinity = true;
+            pts[e].push_back(p); sc[e].push_back(Fe{});
+        }
+        const std::vector<Affine> r = VariableBaseMSM::multi_scalar_mul_batch(*ck.ctx(), ck.curve(), pts, sc);
+        return InputInstance{r[0], r[1], r[2]};
+    }
+private:
+    static Fe mul(const accmsm::hostfp::Modulus &M, const Fe &a, const Fe &b) { Fe r; accmsm::hostfp::mul(M, a.data(), b.data(), r.data()); return r; }
+    static Fe add(const accmsm::hostfp::Modulus &M, const Fe &a, const Fe &b) { Fe r; accmsm::hostfp::add(M, a.data(), b.data(), r.data()); return r; }
+    static Fe canonical(const accmsm::hostfp::Modulus &M, const Fe &a) { const Fe one{1, 0, 0, 0}; return mul(M, a, one); }   // a R * 1 * R^-1
+    static std::vector<Fe> powers(const accmsm::hostfp::Modulus &M, const Fe &x, size_t k) {
+        std::vector<Fe> p(k);
+        if (k) p[0] = Fe{M.one[0], M.one[1], M.one[2], M.one[3]};
+        for (size_t j = 1; j < k; j++) p[j] = mul(M, p[j - 1], x);
+        return p;
     }
 };
 

@@ -91,6 +91,18 @@ def _canon(values) -> np.ndarray:
     return np.array([[(v >> (64 * j)) & 0xFFFFFFFFFFFFFFFF for j in range(4)] for v in values], dtype=np.uint64).reshape(-1, 4)
 
 
+def _canon_mont(field: int, values) -> np.ndarray:
+    """integers -> (n, 4) Montgomery limbs"""
+    return np.array([_int_to_fe(field, v) for v in values], dtype=np.uint64).reshape(-1, 4)
+
+
+def _same_affine(a, b) -> bool:
+    """GroupAffine PartialEq on (xy, inf) pairs: both identity, or the same (x, y)"""
+    if int(a[1]) or int(b[1]):
+        return bool(int(a[1])) == bool(int(b[1]))
+    return np.array_equal(np.asarray(a[0], dtype=np.uint64), np.asarray(b[0], dtype=np.uint64))
+
+
 @dataclass
 class ZkHiding:
     """What a zk opening (MakeZK::Enabled) adds to InnerProductArgPC.open: the random hiding polynomial (<= 2^k
@@ -311,6 +323,97 @@ class ASForHadamardProducts:
         r = None if rand is None else np.array([np.asarray(x, dtype=np.uint64) for x in rand])
         ok, _, _ = ck.bases.ctx.hp_decide(ck.bases, a, b, exp_xy, exp_inf, hiding_index=ck.num_generators, randomness=r)
         return ok
+
+    @staticmethod
+    def prove(ck: CommitterKey, witnesses, instances, mu_fn: Callable, nu_fn: Callable, zk=None):   # :646-813
+        """ASForHadamardProducts::prove over the already padded pairs, inputs first, then old accumulators (the placeholder
+        padding of :676-710 stays with the caller).  witnesses: [(a, b, (r1, r2, r3) | None)], instances: [(C1, C2, C3)] with
+        (xy, inf) points.  zk = (ha, hb, (hr1, hr2, hr3)) from the caller's rng (ha, hb of hp_vec_len = ck.num_generators
+        elements).  The sponge is the callables: mu_fn(hiding_comms | None) -> mu_1 .. mu_{n-1} and nu_fn(low, high) -> nu
+        (Montgomery limbs).  One device session (begin, product_poly_comm, finish) forms the hiding commitments, the
+        product-polynomial commitments and a*, b*; the randomness (App. C.5) is host arithmetic and the new instance (C.6) one
+        3-equation msm_oneshot_batch.  -> (new instance (C1*, C2*, C3*), new witness (a*, b*, rand* | None),
+        proof (hiding_comms | None, low, high))"""
+        from . import scalar_field
+        ctx, f = ck.bases.ctx, scalar_field(ck.curve)
+        m, L, n = _MODULI[f], ck.num_generators, len(witnesses)
+        a = [np.ascontiguousarray(w[0], dtype=np.uint64).reshape(-1, 4)[:L] for w in witnesses]
+        b = [np.ascontiguousarray(w[1], dtype=np.uint64).reshape(-1, 4)[:L] for w in witnesses]
+        ha, hb, hr = (None, None, None) if zk is None else zk
+        sess, hc = ctx.hp_prove_begin(ck.bases, a, b, L, ha, hb, hiding_index=ck.num_generators, hiding_rand=None if hr is None else np.array(hr))
+        try:
+            hiding_comms = None if hc is None else [(hc[0][j], int(hc[1][j])) for j in range(3)]
+            mus = [_fe_to_int(f, x) for x in np.asarray(mu_fn(hiding_comms), dtype=np.uint64).reshape(-1, 4)]
+            mu = [1] + mus + ([mus[0] * mus[-1] % m] if zk is not None else [])
+            (lo, linf), (hi, hinf) = ctx.hp_prove_product_poly_comm(sess, n, _canon_mont(f, mu))
+            low = [(lo[j], int(linf[j])) for j in range(n - 1)]
+            high = [(hi[j], int(hinf[j])) for j in range(n - 1)]
+            nu = np.ascontiguousarray(nu_fn(low, high), dtype=np.uint64).reshape(4)
+        except Exception:
+            try:
+                ctx.hp_prove_abort(sess)
+            except Exception:
+                pass
+            raise
+        a_star, b_star = ctx.hp_prove_finish(sess, nu, L)
+        v = _fe_to_int(f, nu)
+        nus = [pow(v, j, m) for j in range(2 * n - 1)]
+        rand = None
+        if zk is not None:
+            hrs = [_fe_to_int(f, x) for x in hr]
+            rs = [None if w[2] is None else [_fe_to_int(f, x) for x in w[2]] for w in witnesses]
+            mu_n = mu[n]
+            r1 = (mu_n * hrs[0] + sum(mu[i] * nus[i] * rs[i][0] for i in range(n) if rs[i] is not None)) % m
+            r2 = (mu[1] * hrs[1] + sum(nus[j] * rs[n - 1 - j][1] for j in range(n) if rs[n - 1 - j] is not None)) % m
+            r3 = (mu_n * hrs[2] + sum(mu[i] * rs[i][2] for i in range(n) if rs[i] is not None)) * nus[n - 1] % m
+            rand = [_int_to_fe(f, r) for r in (r1, r2, r3)]
+        new_instance = ASForHadamardProducts.combined_commitments(ck, instances, hiding_comms, low, high, mu, v)
+        return new_instance, (a_star, b_star, rand), (hiding_comms, low, high)
+
+    @staticmethod
+    def combined_commitments(ck: CommitterKey, instances, hiding_comms, low, high, mu, nu: int):    # :409-479 (App. C.6)
+        """C1* = [mu_n H1] + sum_i mu_i nu^i C1_i,  C2* = [mu_1 H2] + sum_j nu^j C2_{n-1-j},
+        C3* = sum_j nu^j low_j + sum_j nu^(n+j) high_j + nu^(n-1) ([mu_n H3] + sum_i mu_i C3_i), as ONE msm_oneshot_batch of
+        3 equations padded with (identity, 0) terms.  mu: integers (n, n + 1 with hiding entries), nu: an integer."""
+        from . import scalar_field
+        m = _MODULI[scalar_field(ck.curve)]
+        n = len(instances)
+        nus = [pow(nu, j, m) for j in range(2 * n - 1)]
+        e1 = [(instances[i][0], mu[i] * nus[i]) for i in range(n)]
+        e2 = [(instances[n - 1 - j][1], nus[j]) for j in range(n)]
+        e3 = [(low[j], nus[j]) for j in range(n - 1)] + [(high[j], nus[n + j]) for j in range(n - 1)]
+        e3 += [(instances[i][2], mu[i] * nus[n - 1]) for i in range(n)]
+        if hiding_comms is not None:
+            e1.append((hiding_comms[0], mu[n]))
+            e2.append((hiding_comms[1], mu[1]))
+            e3.append((hiding_comms[2], mu[n] * nus[n - 1]))
+        eqs = [e1, e2, e3]
+        width = max(len(e) for e in eqs)
+        eqs = [e + [((e[0][0][0], 1), 0)] * (width - len(e)) for e in eqs]     # (a point flagged as the identity, 0)
+        pts = np.array([[np.asarray(p[0], dtype=np.uint64) for p, _ in e] for e in eqs])
+        infs = np.array([[int(p[1]) for p, _ in e] for e in eqs], dtype=np.uint8)
+        sc = np.stack([_canon([s % m for _, s in e]) for e in eqs])
+        xy, inf = ck.bases.ctx.msm_oneshot_batch(ck.curve, pts, sc, montgomery=False, infinity=infs)
+        return tuple((xy[j], int(inf[j])) for j in range(3))
+
+    @staticmethod
+    def verify(ck: CommitterKey, instances, new_instance, proof, mu_fn: Callable, nu_fn: Callable) -> bool:   # :815-892
+        """The verifier's O(n) recomputation: mu and nu from the same sponge callables as prove, then C1*, C2*, C3* from the
+        old instances and the proof (one msm_oneshot_batch), accept iff they equal new_instance.  A proof whose shape does not
+        fit n (low / high of n - 1 points each) is rejected."""
+        from . import scalar_field
+        f = scalar_field(ck.curve)
+        m, n = _MODULI[f], len(instances)
+        hiding_comms, low, high = proof
+        if n < 1 or len(low) != n - 1 or len(high) != n - 1 or (hiding_comms is not None and len(hiding_comms) != 3):
+            return False
+        mus = [_fe_to_int(f, x) for x in np.asarray(mu_fn(hiding_comms), dtype=np.uint64).reshape(-1, 4)]
+        if len(mus) != n - 1:
+            return False
+        mu = [1] + mus + ([mus[0] * mus[-1] % m] if hiding_comms is not None else [])
+        nu = _fe_to_int(f, nu_fn(low, high))
+        got = ASForHadamardProducts.combined_commitments(ck, instances, hiding_comms, low, high, mu, nu)
+        return all(_same_affine(g, e) for g, e in zip(got, new_instance))
 
 
 @dataclass

@@ -375,6 +375,35 @@ int accmsm_nark_as_decide(accmsm_ctx *ctx, uint64_t key_handle, uint64_t csr_han
                           size_t hiding_index, const uint64_t *sigmas_mont, const uint64_t *hp_rand_mont, const uint64_t *expected_xy,
                           const uint8_t *expected_inf, int *accept, uint64_t *out_xy, uint8_t *out_inf);
 
+/* ---- ASForHadamardProducts::prove as a session (src/hp_as/mod.rs:646-813; SURVEY.md App. C.1-C.6) -------------------------
+ * The n_in pairs (a_i, b_i) -- inputs first, then old accumulators, after the caller's placeholder padding -- are uploaded
+ * once and stay in HBM until finish; the host keeps the sponge and the O(n) pieces (r1*, r2*, r3*, C1*, C2*, C3*):
+ *     begin(pairs, hiding) -> hiding comms;  mu = sponge(.., hiding comms)
+ *     product_poly_comm(mu) -> low, high;    nu = sponge(.., low, high)
+ *     finish(nu) -> a*, b*
+ * begin: each a_i, b_i holds a_lens[i] / b_lens[i] <= len elements, len <= the key length.  Zero knowledge: hiding_a and
+ *   hiding_b (len x 4 each, both or neither), hiding_rand (r1, r2, r3: 3 x 4) and the generator index hiding_index; begin then
+ *   returns Commit(ha, r1), Commit(hb, r2), Commit(ha o b_0 + a_{n-1} o hb, r3) (3 x 8, 3) from one pass.  The last vector is
+ *   the hiding part of the middle t-vector, which holds only for n_in >= 2 (with n_in = 1 it also carries mu_1^2 ha o hb):
+ *   hiding with n_in = 1 is ACCMSM_E_ARG (the reference's zk padding keeps n >= 2).  Without hiding begin runs no kernel.
+ * product_poly_comm: mu = (mu_0 = 1, mu_1 .. mu_{n-1}) and, with hiding, mu_n = mu_1 mu_{n-1} (n_mu = n_in (+1)); low / high:
+ *   (n_in - 1) x 8 and n_in - 1 flags each, as accmsm_hp_product_poly_comm.
+ * finish: a* = mu_n ha + sum_i mu_i nu^i a_i and b* = mu_1 hb + sum_j nu^j b_{n-1-j} (App. C.5) into a_star / b_star (capacity
+ *   elements each); out_len[0] / out_len[1] receive their lengths, max(a_lens (, len with hiding)) and max(b_lens (, len)).
+ *   finish releases the session, on error too; abort releases it without results.
+ * ACCMSM_E_ARG (the session stays usable unless finish was called): steps out of order, a wrong n_mu, n_in outside
+ * 1..16, one hiding vector without the other, hiding with n_in = 1, a vector longer than len.  An unknown session:
+ * ACCMSM_E_HANDLE.  Calls on the same ctx between the steps do not disturb a session, and several sessions may be live. */
+int accmsm_hp_prove_begin(accmsm_ctx *ctx, uint64_t key_handle, const uint64_t *const *a_vecs, const size_t *a_lens,
+                          const uint64_t *const *b_vecs, const size_t *b_lens, int n_in, size_t len, const uint64_t *hiding_a,
+                          const uint64_t *hiding_b, size_t hiding_index, const uint64_t *hiding_rand_mont, uint64_t *hiding_comm_xy,
+                          uint8_t *hiding_comm_inf, uint64_t *session);
+int accmsm_hp_prove_product_poly_comm(accmsm_ctx *ctx, uint64_t session, const uint64_t *mu_mont, size_t n_mu, uint64_t *low_xy,
+                                      uint8_t *low_inf, uint64_t *high_xy, uint8_t *high_inf);
+int accmsm_hp_prove_finish(accmsm_ctx *ctx, uint64_t session, const uint64_t nu_mont[4], uint64_t *a_star, uint64_t *b_star,
+                           size_t capacity, size_t *out_len);
+int accmsm_hp_prove_abort(accmsm_ctx *ctx, uint64_t session);
+
 #ifdef __cplusplus
 }
 #endif
