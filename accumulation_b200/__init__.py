@@ -544,6 +544,45 @@ class Context:
     def hp_prove_abort(self, session: int):
         self._check(self._lib.accmsm_hp_prove_abort(self._h, C.c_uint64(session)), "hp_prove_abort")
 
+    def nark_as_prove_begin(self, bases: "Bases", csr: int, inputs, blinded_witnesses, acc_witnesses, acc_a, acc_b, zk=None,
+                            hiding_index: int = 0, n_input: Optional[int] = None):
+        """ASForR1CSNark::prove, first step (SURVEY App. C.12): an hp_prove session whose first pairs are A (x_i || w'_i),
+        B (x_i || w'_i) of the fresh inputs (one row-kernel launch), then the accumulators' (a*_j, b*_j).  zk = (r_x, r_w, ha, hb,
+        rand) with rand = (sigma_rA, sigma_rB, sigma_rC, r1, r2, r3): the same launch forms M (r_x || r_w) and one 6-job pass
+        returns H1, H2, H3, comm_rA, comm_rB, comm_rC.  Continue with hp_prove_product_poly_comm and nark_as_prove_finish
+        n_input: the index's input length, needed (for the column check) when there is neither a fresh input nor zk
+        -> (session, (xy (6, 8), inf (6,)) | None)"""
+        xs = [_u64(v).reshape(-1, 4) for v in inputs]
+        ws = [_u64(v).reshape(-1, 4) for v in blinded_witnesses]
+        aw = [_u64(v).reshape(-1, 4) for v in acc_witnesses]
+        aa = [_u64(v).reshape(-1, 4) for v in acc_a]
+        bb = [_u64(v).reshape(-1, 4) for v in acc_b]
+        if n_input is None:
+            n_input = xs[0].shape[0] if xs else (_u64(zk[0]).reshape(-1, 4).shape[0] if zk is not None else 0)
+        n_witness = ws[0].shape[0] if ws else (aw[0].shape[0] if aw else 0)
+        al = np.array([v.shape[0] for v in aa] or [0], dtype=np.uint64)
+        bl = np.array([v.shape[0] for v in bb] or [0], dtype=np.uint64)
+        rx, rw, ha, hb, rand = (None,) * 5 if zk is None else (_u64(zk[0]).reshape(-1, 4), _u64(zk[1]).reshape(-1, 4), _u64(zk[2]).reshape(-1, 4),
+                                                            _u64(zk[3]).reshape(-1, 4), _u64(zk[4]).reshape(6, 4))
+        out, oinf = np.zeros((6, 8), dtype=np.uint64), np.zeros(6, dtype=np.uint8)
+        sess = C.c_uint64(0)
+        self._check(self._lib.accmsm_nark_as_prove_begin(
+            self._h, C.c_uint64(bases.handle), C.c_uint64(csr), C.c_int(len(xs)), self._ptrs(xs), C.c_size_t(n_input), self._ptrs(ws),
+            C.c_size_t(n_witness), C.c_int(len(aa)), self._ptrs(aw), self._ptrs(aa), _p(al), self._ptrs(bb), _p(bl), _p(rx), _p(rw), _p(ha),
+            _p(hb), C.c_size_t(hiding_index), _p(rand), _p(out), _p(oinf), C.byref(sess)), "nark_as_prove_begin")
+        return int(sess.value), (None if zk is None else (out, oinf))
+
+    def nark_as_prove_finish(self, session: int, nu, beta, capacity: int, n_witness: int):
+        """last step: a*, b* as hp_prove_finish and w* = sum_k beta_k w_k (w'_i, then w*_j, then r_w with zk; beta_0 = 1
+        included); releases the session (on error too) -> (a*, b*, w*)"""
+        beta = _u64(beta).reshape(-1, 4)
+        a, b = np.empty((capacity, 4), dtype=np.uint64), np.empty((capacity, 4), dtype=np.uint64)
+        w = np.empty((n_witness, 4), dtype=np.uint64)
+        olen = (C.c_size_t * 2)()
+        self._check(self._lib.accmsm_nark_as_prove_finish(self._h, C.c_uint64(session), _p(_u64(nu)), _p(beta), C.c_size_t(beta.shape[0]),
+                                                          _p(a), _p(b), C.c_size_t(capacity), olen, _p(w)), "nark_as_prove_finish")
+        return a[: olen[0]], b[: olen[1]], w
+
     # ---- field-vector kernels
     def compute_coeffs(self, field: int, challenges_mont):
         ch = _u64(challenges_mont).reshape(-1, 4)

@@ -20,6 +20,7 @@ SYMBOLS = [
     "accmsm_hp_decide", "accmsm_hp_decide_partial_dev", "accmsm_hp_product_poly_comm", "accmsm_hp_product_poly_comm_partial_dev", "accmsm_csr_matvec_commit_partial_dev", "accmsm_register_csr", "accmsm_release_csr", "accmsm_csr_matvec_commit",
     "accmsm_nark_prove_zk", "accmsm_nark_verify", "accmsm_nark_as_decide",
     "accmsm_hp_prove_begin", "accmsm_hp_prove_product_poly_comm", "accmsm_hp_prove_finish", "accmsm_hp_prove_abort",
+    "accmsm_nark_as_prove_begin", "accmsm_nark_as_prove_finish",
     "accmsm_vec_hadamard", "accmsm_vec_scale", "accmsm_vec_lincomb", "accmsm_vec_tvecs", "accmsm_csr_matvec",
 ]
 

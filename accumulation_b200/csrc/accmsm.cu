@@ -999,8 +999,15 @@ int group_hp_prove_begin(accmsm_ctx *g, uint64_t key_handle, const uint64_t *con
 int group_hp_prove_ppc(accmsm_ctx *g, uint64_t session, const uint64_t *mu_mont, size_t n_mu, uint64_t *low_xy, uint8_t *low_inf,
                        uint64_t *high_xy, uint8_t *high_inf);
 int group_hp_prove_finish(accmsm_ctx *g, uint64_t session, const uint64_t nu_mont[4], uint64_t *a_star, uint64_t *b_star, size_t capacity,
-                          size_t *out_len);
+                          size_t *out_len, bool nark_as = false, const uint64_t *beta_mont = nullptr, size_t n_beta = 0,
+                          uint64_t *w_star = nullptr);
 int group_hp_prove_abort(accmsm_ctx *g, uint64_t session);
+// ASForR1CSNark::prove sessions: an hp session per child over its rows of the key and the matrices
+int group_nark_as_prove_begin(accmsm_ctx *g, uint64_t key_handle, uint64_t csr_handle, int n_fresh, const uint64_t *const *inputs,
+                              size_t n_input, const uint64_t *const *witnesses, size_t n_witness, int n_acc, const uint64_t *const *acc_w,
+                              const uint64_t *const *acc_a, const size_t *acc_a_lens, const uint64_t *const *acc_b, const size_t *acc_b_lens,
+                              const uint64_t *r_input, const uint64_t *r_witness, const uint64_t *hiding_a, const uint64_t *hiding_b,
+                              size_t hiding_index, const uint64_t *tails_mont, uint64_t *comm_xy, uint8_t *comm_inf, uint64_t *session);
 // IpaPC::open sessions sharded cyclically across the children of a group (multi_api.inc).  GROUP_IPA_UNSHARDED: the
 // opening is too small to shard / the id is not a sharded session, and child 0 serves the call as before.
 constexpr int GROUP_IPA_UNSHARDED = 1;

@@ -289,4 +289,50 @@ __global__ void __launch_bounds__(256) k_nark_rows(CsrMats mats, uint32_t n_rows
     }
 }
 
+// entries [e0, e1) of one CSR row against z = x || w
+template <int FIELD>
+ACC_D fe_t csr_row_dot(const uint32_t *__restrict__ cols, const uint8_t *__restrict__ coeffs, uint32_t e0, uint32_t e1,
+                       const uint8_t *__restrict__ x, uint32_t n_input, const uint8_t *__restrict__ w) {
+    using F = Fp<FIELD>;
+    const fe_t one = F::one();
+    fe_t acc = F::zero();
+    for (uint32_t e = e0; e < e1; e++) {
+        const uint32_t col = cols[e];
+        const fe_t cf = load_fe_nc(coeffs + (size_t)e * 32);
+        const fe_t z = col < n_input ? load_fe(x + (size_t)col * 32) : load_fe(w + (size_t)(col - n_input) * 32);
+        acc = F::add(acc, F::eq(cf, one) ? z : F::mul(z, cf));   // coeff.is_one() fast path (:459)
+    }
+    return acc;
+}
+
+// ASForR1CSNark::prove rows (src/r1cs_nark_as/mod.rs:316-420; SURVEY.md App. C.12 steps 1 and 3): one thread per constraint
+// row.  For every fresh input i it walks row r of A and B over x_i || w'_i (inputs: n_fresh x n_input, witnesses: n_fresh x
+// n_witness, packed) and stores A (x_i || w'_i) and B (x_i || w'_i) at position r of the hp pair vectors a_i = pairs + i
+// pair_stride and b_i = pairs + (n_fresh + i) pair_stride.  The inputs are looped inside the thread, re-reading the row's
+// (col, coeff) entries from L1, so the registers do not grow with n_fresh.  ZK: it also walks row r of A, B and C over
+// r_x || r_w and stores M (r_x || r_w) into rows 3, 4, 5 of the pass's scalar rows (out + (3 + m) row_stride).
+template <int FIELD, bool ZK>
+__global__ void __launch_bounds__(256) k_nark_as_rows(CsrMats mats, uint32_t n_rows, const uint8_t *__restrict__ inputs,
+                                                       uint32_t n_input, const uint8_t *__restrict__ witnesses, uint32_t n_witness,
+                                                       uint32_t n_fresh, uint8_t *__restrict__ pairs, size_t pair_stride,
+                                                       const uint8_t *__restrict__ r_input, const uint8_t *__restrict__ r_witness,
+                                                       uint8_t *__restrict__ out, size_t row_stride) {
+    uint32_t r = blockIdx.x * blockDim.x + threadIdx.x;
+    if (r >= n_rows) return;
+#pragma unroll      // static indices into the CsrMats parameter: a dynamic one copies it to the stack
+    for (int mi = 0; mi < (ZK ? 3 : 2); mi++) {
+        const uint32_t e0 = mats.row_ptr[mi][r], e1 = mats.row_ptr[mi][r + 1];
+        if (mi < 2) {
+#pragma unroll 1
+            for (uint32_t i = 0; i < n_fresh; i++) {
+                const fe_t t = csr_row_dot<FIELD>(mats.cols[mi], mats.coeffs[mi], e0, e1, inputs + (size_t)i * n_input * 32, n_input,
+                                                  witnesses + (size_t)i * n_witness * 32);
+                store_fe(pairs + (size_t)(mi * n_fresh + i) * pair_stride + (size_t)r * 32, t);
+            }
+        }
+        if (ZK) store_fe(out + (size_t)(3 + mi) * row_stride + (size_t)r * 32,
+                         csr_row_dot<FIELD>(mats.cols[mi], mats.coeffs[mi], e0, e1, r_input, n_input, r_witness));
+    }
+}
+
 }  // namespace accmsm

@@ -13,8 +13,9 @@
 //   r1cs_nark: Matrix<F> = Vec<Vec<(F, usize)>>, matrix_vec_mul,       r1cs_nark::{Matrix, matrix_vec_mul, IndexMatrices}
 //              R1CSNark::prove (zk first message) / verify             IndexMatrices::{matvec_commit, prove_zk, verify}
 //                                        (src/r1cs_nark_as/r1cs_nark/mod.rs:183-419, 443-462)
-//   r1cs_nark_as: AccumulatorInstance, AccumulatorWitness, decide       r1cs_nark_as::{AccumulatorInstance, AccumulatorWitness, decide}
-//                                        (src/r1cs_nark_as/data_structures.rs:156-227, src/r1cs_nark_as/mod.rs:1031-1112)
+//   r1cs_nark_as: AccumulatorInstance, AccumulatorWitness, prove,       r1cs_nark_as::{AccumulatorInstance, AccumulatorWitness, prove,
+//                 decide                                               decide}
+//                                        (src/r1cs_nark_as/data_structures.rs:156-227, src/r1cs_nark_as/mod.rs:713-926, 1031-1112)
 // Every call computes on the GPU; there is no CPU path.  ark's commit is infallible -> failures throw AccmsmError
 // (the Rust wrapper panics / maps to PCError at the same places).
 #pragma once
@@ -362,7 +363,6 @@ struct ASForHadamardProducts {
     static ProveOutput prove(const CommitterKey &ck, const std::vector<InputWitness> &witnesses, const std::vector<InputInstance> &instances,
                              const MuOf &mu_of, const NuOf &nu_of, const std::optional<HidingVecs> &zk = std::nullopt) {
         const size_t n = witnesses.size(), L = ck.supported_num_elems();
-        const accmsm::hostfp::Modulus &M = accmsm::hostfp::modulus(scalar_field(ck.curve()));
         if (zk && !ck.has_hiding()) throw AccmsmError("prove: the key has no hiding generator");
         if (instances.size() != n) throw AccmsmError("prove: one instance per witness");
         std::vector<const uint64_t *> ap, bp; std::vector<size_t> al, bl;
@@ -383,42 +383,62 @@ struct ASForHadamardProducts {
         ck.ctx()->check(accmsm_hp_prove_begin(c, ck.handle(), ap.data(), al.data(), bp.data(), bl.data(), (int)n, L,
                                               zk ? (L ? ha[0].data() : zero[0].data()) : nullptr, zk ? (L ? hb[0].data() : zero[0].data()) : nullptr,
                                               ck.hiding_index(), zk ? hr : nullptr, hxy, hinf, &sess), "hp_prove_begin");
+        std::optional<std::array<Affine, 3>> hiding_comms;
+        if (zk) hiding_comms = std::array<Affine, 3>{affine_from(hxy, hinf[0]), affine_from(hxy + 8, hinf[1]), affine_from(hxy + 16, hinf[2])};
+        std::vector<std::optional<Randomness>> rands;
+        for (const auto &w : witnesses) rands.push_back(w.randomness);
+        return run_session(ck, sess, hiding_comms, rands, instances, mu_of, nu_of, zk ? std::optional<Randomness>(zk->randomness) : std::nullopt,
+                           [&](const Fe &nu, const InputInstance &, std::vector<Fe> &a_star, std::vector<Fe> &b_star) {
+            a_star.resize(L); b_star.resize(L);
+            size_t olen[2] = {0, 0};
+            ck.ctx()->check(accmsm_hp_prove_finish(c, sess, nu.data(), L ? a_star[0].data() : nullptr, L ? b_star[0].data() : nullptr, L, olen),
+                            "hp_prove_finish");
+            a_star.resize(olen[0]); b_star.resize(olen[1]);
+        });
+    }
+    // The steps of an hp-prove session after its begin, shared by prove and r1cs_nark_as::prove: mu from the hiding commitments,
+    // product_poly_comm, nu, the new instance (C.6), then finish(nu, new instance, a*, b*), the caller's last call on the session,
+    // and the randomness (App. C.5) on the host.  rands: the pairs' randomness; hiding_rand: with zk.  The session is aborted if a
+    // step up to finish fails (after finish has released it the abort is a harmless ACCMSM_E_HANDLE).
+    using Finish = std::function<void(const Fe &nu, const InputInstance &new_instance, std::vector<Fe> &a_star, std::vector<Fe> &b_star)>;
+    static ProveOutput run_session(const CommitterKey &ck, uint64_t sess, const std::optional<std::array<Affine, 3>> &hiding_comms,
+                                   const std::vector<std::optional<Randomness>> &rands, const std::vector<InputInstance> &instances,
+                                   const MuOf &mu_of, const NuOf &nu_of, const std::optional<Randomness> &hiding_rand, const Finish &finish) {
+        const size_t n = instances.size();
+        const accmsm::hostfp::Modulus &M = accmsm::hostfp::modulus(scalar_field(ck.curve()));
+        accmsm_ctx *c = ck.ctx()->raw();
         ProveOutput out;
+        out.proof.hiding_comms = hiding_comms;
         std::vector<Fe> mu(1, Fe{M.one[0], M.one[1], M.one[2], M.one[3]});
+        Fe nu;
         try {
-            if (zk) out.proof.hiding_comms = std::array<Affine, 3>{affine_from(hxy, hinf[0]), affine_from(hxy + 8, hinf[1]), affine_from(hxy + 16, hinf[2])};
             const std::vector<Fe> mus = mu_of(out.proof.hiding_comms);
             if (mus.size() + 1 != n) throw AccmsmError("prove: mu_of must return n - 1 challenges");
             mu.insert(mu.end(), mus.begin(), mus.end());
-            if (zk) { Fe mn; accmsm::hostfp::mul(M, mu[1].data(), mu[n - 1].data(), mn.data()); mu.push_back(mn); }
+            if (hiding_comms) mu.push_back(mul(M, mu[1], mu[n - 1]));
             std::vector<uint64_t> lo(8 * n), hi(8 * n); std::vector<uint8_t> li(n), hinf2(n);
             ck.ctx()->check(accmsm_hp_prove_product_poly_comm(c, sess, mu[0].data(), mu.size(), lo.data(), li.data(), hi.data(), hinf2.data()),
                             "hp_prove_product_poly_comm");
             for (size_t j = 0; j + 1 < n; j++) { out.proof.low.push_back(affine_from(&lo[8 * j], li[j])); out.proof.high.push_back(affine_from(&hi[8 * j], hinf2[j])); }
+            nu = nu_of(out.proof.low, out.proof.high);
+            out.instance = combined_commitments(ck, instances, out.proof, mu, nu);
+            finish(nu, out.instance, out.witness.a_vec, out.witness.b_vec);
         } catch (...) {
             accmsm_hp_prove_abort(c, sess);
             throw;
         }
-        const Fe nu = nu_of(out.proof.low, out.proof.high);
-        std::vector<Fe> a_star(L), b_star(L);
-        size_t olen[2] = {0, 0};
-        ck.ctx()->check(accmsm_hp_prove_finish(c, sess, nu.data(), L ? a_star[0].data() : nullptr, L ? b_star[0].data() : nullptr, L, olen),
-                        "hp_prove_finish");
-        a_star.resize(olen[0]); b_star.resize(olen[1]);
-        out.witness.a_vec = std::move(a_star); out.witness.b_vec = std::move(b_star);
         const std::vector<Fe> nus = powers(M, nu, 2 * n - 1);
-        if (zk) {       // App. C.5; absent randomness entries add nothing
-            Fe r1 = mul(M, mu[n], zk->randomness.rand_1), r2 = mul(M, mu[1], zk->randomness.rand_2), r3 = mul(M, mu[n], zk->randomness.rand_3);
+        if (hiding_rand) {       // App. C.5; absent randomness entries add nothing
+            Fe r1 = mul(M, mu[n], hiding_rand->rand_1), r2 = mul(M, mu[1], hiding_rand->rand_2), r3 = mul(M, mu[n], hiding_rand->rand_3);
             for (size_t i = 0; i < n; i++) {
-                if (const auto &r = witnesses[i].randomness) {
+                if (const auto &r = rands[i]) {
                     r1 = add(M, r1, mul(M, mul(M, mu[i], nus[i]), r->rand_1));
                     r3 = add(M, r3, mul(M, mu[i], r->rand_3));
                 }
-                if (const auto &r = witnesses[n - 1 - i].randomness) r2 = add(M, r2, mul(M, nus[i], r->rand_2));
+                if (const auto &r = rands[n - 1 - i]) r2 = add(M, r2, mul(M, nus[i], r->rand_2));
             }
             out.witness.randomness = Randomness{r1, r2, mul(M, r3, nus[n - 1])};
         }
-        out.instance = combined_commitments(ck, instances, out.proof, mu, nu);
         return out;
     }
     // verify (:815-892): mu and nu from the same sponge, C1*, C2*, C3* recomputed from the old instances and the proof; accept iff
@@ -466,7 +486,7 @@ struct ASForHadamardProducts {
         const std::vector<Affine> r = VariableBaseMSM::multi_scalar_mul_batch(*ck.ctx(), ck.curve(), pts, sc);
         return InputInstance{r[0], r[1], r[2]};
     }
-private:
+    // host field helpers (Montgomery images), also used by r1cs_nark_as::prove
     static Fe mul(const accmsm::hostfp::Modulus &M, const Fe &a, const Fe &b) { Fe r; accmsm::hostfp::mul(M, a.data(), b.data(), r.data()); return r; }
     static Fe add(const accmsm::hostfp::Modulus &M, const Fe &a, const Fe &b) { Fe r; accmsm::hostfp::add(M, a.data(), b.data(), r.data()); return r; }
     static Fe canonical(const accmsm::hostfp::Modulus &M, const Fe &a) { const Fe one{1, 0, 0, 0}; return mul(M, a, one); }   // a R * 1 * R^-1
@@ -519,6 +539,7 @@ public:
     ~IndexMatrices() { accmsm_release_csr(ck_.ctx()->raw(), handle_); }
     uint64_t handle() const { return handle_; }
     const CommitterKey &ck() const { return ck_; }
+    size_t n_rows() const { return n_rows_; }
     std::optional<size_t> num_instance_variables() const { return num_instance_variables_; }
     // z_M = M (input || witness), comm_M = Commit(z_M, blinder_M)   (prove :183-185 + :216-218; decide src/r1cs_nark_as/mod.rs:1052-1097)
     std::pair<std::vector<std::vector<Fe>>, std::vector<Affine>> matvec_commit(const std::vector<Fe> &input, const std::vector<Fe> &witness,
@@ -590,6 +611,158 @@ struct AccumulatorWitness {
     ASForHadamardProducts::InputWitness hp_witness;
     std::optional<AccumulatorWitnessRandomness> randomness;
 };
+// ASForR1CSNark::prove (src/r1cs_nark_as/mod.rs:713-926; SURVEY.md App. C.12).  A fresh input is x and its NARK proof (first
+// message of 3 points, or 8 with zk; the blinded witness w'; the sigmas (sigma_A, sigma_B, sigma_C, sigma_o) with zk).  The
+// sponge is the callables: gamma_of(first_msg) for a zk proof, mu_of / nu_of as in ASForHadamardProducts::prove, and
+// beta_of(new hp instance, randomness comms) -> beta_1 .. beta_{n-1} (beta_n too with zk), n = fresh inputs + old accumulators;
+// with zk n >= 2 (the caller pads, src/hp_as/mod.rs:676-710).  One device session (accmsm_nark_as_prove_begin, product_poly_comm,
+// accmsm_nark_as_prove_finish) forms the fresh mat-vecs, the randomness and hp hiding commitments, the hp proof, a*, b* and w*;
+// its hp part is ASForHadamardProducts::run_session.  The blinded commitments of the zk inputs are one batched MSM (4 equations
+// each), comm_A*, comm_B*, comm_C* another (3 equations), and x*, sigma* host arithmetic.
+struct FreshInput { std::vector<Fe> r1cs_input; std::vector<Affine> first_msg; std::vector<Fe> blinded_witness; std::optional<std::array<Fe, 4>> sigmas; };
+struct ProverRandomness {                    // the caller's rng (:366-420): r_x, r_w, sigma_rA, sigma_rB, sigma_rC and the hp hiding vectors
+    std::vector<Fe> r_input, r_witness;
+    std::array<Fe, 3> sigma_r;
+    ASForHadamardProducts::HidingVecs hp;    // n_rows elements each
+};
+struct Proof { ASForHadamardProducts::Proof hp_proof; std::optional<std::array<Affine, 3>> randomness_comms; };
+struct ProveOutput { AccumulatorInstance instance; AccumulatorWitness witness; Proof proof; };
+using GammaOf = std::function<Fe(const std::vector<Affine> &first_msg)>;
+using BetaOf = std::function<std::vector<Fe>(const ASForHadamardProducts::InputInstance &hp_instance,
+                                             const std::optional<std::array<Affine, 3>> &randomness_comms)>;
+inline ProveOutput prove(const r1cs_nark::IndexMatrices &index, const std::vector<FreshInput> &inputs,
+                         const std::vector<std::pair<AccumulatorInstance, AccumulatorWitness>> &old_accumulators, const GammaOf &gamma_of,
+                         const ASForHadamardProducts::MuOf &mu_of, const ASForHadamardProducts::NuOf &nu_of, const BetaOf &beta_of,
+                         const std::optional<ProverRandomness> &zk = std::nullopt) {
+    using HP = ASForHadamardProducts;
+    const CommitterKey &ck = index.ck();
+    const accmsm::hostfp::Modulus &M = accmsm::hostfp::modulus(scalar_field(ck.curve()));
+    const Fe one{M.one[0], M.one[1], M.one[2], M.one[3]};
+    const size_t n_f = inputs.size(), n_a = old_accumulators.size(), n = n_f + n_a, L = index.n_rows();
+    if (n == 0) throw AccmsmError("r1cs_nark_as::prove: no input");
+    if (zk && !ck.has_hiding()) throw AccmsmError("r1cs_nark_as::prove: the key has no hiding generator");
+    const size_t n_input = n_f ? inputs[0].r1cs_input.size() : old_accumulators[0].first.r1cs_input.size();
+    const size_t n_witness = n_f ? inputs[0].blinded_witness.size() : old_accumulators[0].second.r1cs_blinded_witness.size();
+    // step 2: blinded commitments comm_M + gamma comm_rM and comm_C + gamma comm_1 + gamma^2 comm_2, one batched MSM
+    std::vector<std::vector<Affine>> pts;
+    std::vector<std::vector<Fe>> sc;
+    for (const auto &in : inputs) {
+        if (!in.sigmas) continue;
+        if (in.first_msg.size() != 8) throw AccmsmError("r1cs_nark_as::prove: a zk first message has 8 commitments");
+        const auto &fm = in.first_msg;
+        const Fe g = gamma_of(fm), g2 = HP::mul(M, g, g), c1 = HP::canonical(M, one);
+        for (int j = 0; j < 3; j++) {
+            Affine pad = fm[j]; pad.infinity = true;       // (a point flagged as the identity, 0)
+            pts.push_back({fm[j], fm[3 + j], pad}); sc.push_back({c1, HP::canonical(M, g), Fe{}});
+        }
+        pts.push_back({fm[2], fm[6], fm[7]}); sc.push_back({c1, HP::canonical(M, g), HP::canonical(M, g2)});
+    }
+    const std::vector<Affine> comb = pts.empty() ? std::vector<Affine>{} : VariableBaseMSM::multi_scalar_mul_batch(*ck.ctx(), ck.curve(), pts, sc);
+    std::vector<std::array<Affine, 4>> blinded;
+    for (size_t i = 0, k = 0; i < n_f; i++) {
+        const auto &fm = inputs[i].first_msg;
+        if (inputs[i].sigmas) { blinded.push_back({comb[4 * k], comb[4 * k + 1], comb[4 * k + 2], comb[4 * k + 3]}); k++; }
+        else {
+            if (fm.size() < 3) throw AccmsmError("r1cs_nark_as::prove: a first message has 3 commitments");
+            blinded.push_back({fm[0], fm[1], fm[2], fm[2]});
+        }
+    }
+    // step 3: hp inputs, fresh first
+    std::vector<HP::InputInstance> hp_insts;
+    std::vector<std::optional<HP::Randomness>> hp_rands;
+    for (size_t i = 0; i < n_f; i++) {
+        hp_insts.push_back({blinded[i][0], blinded[i][1], blinded[i][3]});
+        const auto &s = inputs[i].sigmas;
+        hp_rands.push_back(s ? std::optional<HP::Randomness>(HP::Randomness{(*s)[0], (*s)[1], (*s)[3]}) : std::nullopt);
+    }
+    for (const auto &acc : old_accumulators) { hp_insts.push_back(acc.first.hp_instance); hp_rands.push_back(acc.second.hp_witness.randomness); }
+    // steps 1 and 3-4 on the device
+    auto ptr = [](const std::vector<Fe> &v) { return v.empty() ? nullptr : v[0].data(); };
+    std::vector<const uint64_t *> xp, wp, awp, ap, bp; std::vector<size_t> al, bl;
+    for (const auto &in : inputs) {
+        if (in.r1cs_input.size() != n_input || in.blinded_witness.size() != n_witness) throw AccmsmError("r1cs_nark_as::prove: input lengths differ");
+        xp.push_back(ptr(in.r1cs_input)); wp.push_back(ptr(in.blinded_witness));
+    }
+    for (const auto &acc : old_accumulators) {
+        if (acc.second.r1cs_blinded_witness.size() != n_witness) throw AccmsmError("r1cs_nark_as::prove: witness lengths differ");
+        const auto &hw = acc.second.hp_witness;
+        awp.push_back(ptr(acc.second.r1cs_blinded_witness)); ap.push_back(ptr(hw.a_vec)); al.push_back(hw.a_vec.size());
+        bp.push_back(ptr(hw.b_vec)); bl.push_back(hw.b_vec.size());
+    }
+    const std::vector<Fe> zero(1);             // zk arguments are all given: an empty one still needs a pointer
+    auto zptr = [&](const std::vector<Fe> &v) { return v.empty() ? zero[0].data() : v[0].data(); };
+    std::vector<Fe> ha, hb;
+    uint64_t rand[24], bxy[48], sess = 0; uint8_t binf[6] = {0, 0, 0, 0, 0, 0};
+    if (zk) {
+        ha = zk->hp.a_vec; hb = zk->hp.b_vec; ha.resize(L); hb.resize(L);
+        const Fe *r[6] = {&zk->sigma_r[0], &zk->sigma_r[1], &zk->sigma_r[2], &zk->hp.randomness.rand_1, &zk->hp.randomness.rand_2, &zk->hp.randomness.rand_3};
+        for (int j = 0; j < 6; j++) std::memcpy(rand + 4 * j, r[j]->data(), 32);
+    }
+    accmsm_ctx *c = ck.ctx()->raw();
+    ck.ctx()->check(accmsm_nark_as_prove_begin(c, ck.handle(), index.handle(), (int)n_f, xp.data(), n_input, wp.data(), n_witness, (int)n_a,
+                                               awp.data(), ap.data(), al.data(), bp.data(), bl.data(), zk ? zptr(zk->r_input) : nullptr,
+                                               zk ? zptr(zk->r_witness) : nullptr, zk ? zptr(ha) : nullptr, zk ? zptr(hb) : nullptr,
+                                               ck.hiding_index(), zk ? rand : nullptr, bxy, binf, &sess), "nark_as_prove_begin");
+    std::optional<std::array<Affine, 3>> hiding_comms, comm_r;
+    if (zk) {
+        hiding_comms = std::array<Affine, 3>{affine_from(bxy, binf[0]), affine_from(bxy + 8, binf[1]), affine_from(bxy + 16, binf[2])};
+        comm_r = std::array<Affine, 3>{affine_from(bxy + 24, binf[3]), affine_from(bxy + 32, binf[4]), affine_from(bxy + 40, binf[5])};
+    }
+    std::vector<Fe> beta(1, one), w_star(n_witness);
+    HP::ProveOutput hp = HP::run_session(ck, sess, hiding_comms, hp_rands, hp_insts, mu_of, nu_of,
+                                         zk ? std::optional<HP::Randomness>(zk->hp.randomness) : std::nullopt,
+                                         [&](const Fe &nu, const HP::InputInstance &hp_inst, std::vector<Fe> &a_star, std::vector<Fe> &b_star) {
+        const std::vector<Fe> b = beta_of(hp_inst, comm_r);     // step 5: beta after the hp proof
+        beta.insert(beta.end(), b.begin(), b.end());
+        a_star.resize(L); b_star.resize(L);
+        size_t olen[2] = {0, 0};
+        ck.ctx()->check(accmsm_nark_as_prove_finish(c, sess, nu.data(), beta[0].data(), beta.size(), L ? a_star[0].data() : nullptr,
+                                                    L ? b_star[0].data() : nullptr, L, olen, n_witness ? w_star[0].data() : nullptr),
+                        "nark_as_prove_finish");
+        a_star.resize(olen[0]); b_star.resize(olen[1]);
+    });
+    // steps 6-7 on the host: fresh inputs, then accumulators, then (zk) the randomness
+    std::vector<const std::vector<Fe> *> xs;
+    std::vector<std::array<Affine, 3>> comms;
+    std::vector<std::optional<std::array<Fe, 3>>> sigs;
+    for (size_t i = 0; i < n_f; i++) {
+        xs.push_back(&inputs[i].r1cs_input);
+        comms.push_back({blinded[i][0], blinded[i][1], blinded[i][2]});
+        const auto &s = inputs[i].sigmas;
+        sigs.push_back(s ? std::optional<std::array<Fe, 3>>(std::array<Fe, 3>{(*s)[0], (*s)[1], (*s)[2]}) : std::nullopt);
+    }
+    for (const auto &acc : old_accumulators) {
+        xs.push_back(&acc.first.r1cs_input);
+        comms.push_back({acc.first.comm_a, acc.first.comm_b, acc.first.comm_c});
+        const auto &r = acc.second.randomness;
+        sigs.push_back(r ? std::optional<std::array<Fe, 3>>(std::array<Fe, 3>{r->sigma_a, r->sigma_b, r->sigma_c}) : std::nullopt);
+    }
+    if (zk) { xs.push_back(&zk->r_input); comms.push_back(*comm_r); sigs.push_back(zk->sigma_r); }
+    ProveOutput out;
+    out.instance.r1cs_input.assign(n_input, Fe{});
+    for (size_t k = 0; k < xs.size(); k++) {
+        if (xs[k]->size() != n_input) throw AccmsmError("r1cs_nark_as::prove: r1cs_input lengths differ");
+        for (size_t j = 0; j < n_input; j++) out.instance.r1cs_input[j] = HP::add(M, out.instance.r1cs_input[j], HP::mul(M, beta[k], (*xs[k])[j]));
+    }
+    std::vector<std::vector<Affine>> cp(3);
+    std::vector<std::vector<Fe>> cs(3);
+    for (size_t k = 0; k < comms.size(); k++) for (int m = 0; m < 3; m++) { cp[m].push_back(comms[k][m]); cs[m].push_back(HP::canonical(M, beta[k])); }
+    const std::vector<Affine> cstar = VariableBaseMSM::multi_scalar_mul_batch(*ck.ctx(), ck.curve(), cp, cs);
+    out.instance.comm_a = cstar[0]; out.instance.comm_b = cstar[1]; out.instance.comm_c = cstar[2];
+    out.instance.hp_instance = hp.instance;
+    bool any_sigma = false;
+    std::array<Fe, 3> sig{};
+    for (size_t k = 0; k < sigs.size(); k++) if (sigs[k]) {
+        any_sigma = true;
+        for (int m = 0; m < 3; m++) sig[m] = HP::add(M, sig[m], HP::mul(M, beta[k], (*sigs[k])[m]));
+    }
+    if (any_sigma) out.witness.randomness = AccumulatorWitnessRandomness{sig[0], sig[1], sig[2]};
+    out.witness.r1cs_blinded_witness = std::move(w_star);
+    out.witness.hp_witness = std::move(hp.witness);
+    out.proof = Proof{std::move(hp.proof), comm_r};
+    return out;
+}
+
 // ASForR1CSNark::decide (src/r1cs_nark_as/mod.rs:1031-1112): t_M = M (r1cs_input || r1cs_blinded_witness); accept iff
 // Commit(t_M, sigma_M) == comm_M for M = A, B, C and hp_as::decide(ck, hp_instance, hp_witness), in ONE library call (one
 // vector launch, the six commitments in one pass).  An r1cs_input whose length differs from the index's is rejected here.

@@ -96,6 +96,20 @@ def _canon_mont(field: int, values) -> np.ndarray:
     return np.array([_int_to_fe(field, v) for v in values], dtype=np.uint64).reshape(-1, 4)
 
 
+def _oneshot_equations(ck: CommitterKey, eqs) -> list:
+    """sum_k s_k P_k for every equation [(P_k as (xy, inf), integer s_k)], all of them in ONE msm_oneshot_batch, the shorter ones
+    padded with (identity, 0) terms -> [(xy, inf)]"""
+    from . import scalar_field
+    m = _MODULI[scalar_field(ck.curve)]
+    width = max(len(e) for e in eqs)
+    eqs = [e + [((e[0][0][0], 1), 0)] * (width - len(e)) for e in eqs]     # (a point flagged as the identity, 0)
+    pts = np.array([[np.asarray(p[0], dtype=np.uint64) for p, _ in e] for e in eqs])
+    infs = np.array([[int(p[1]) for p, _ in e] for e in eqs], dtype=np.uint8)
+    sc = np.stack([_canon([s % m for _, s in e]) for e in eqs])
+    xy, inf = ck.bases.ctx.msm_oneshot_batch(ck.curve, pts, sc, montgomery=False, infinity=infs)
+    return [(xy[j], int(inf[j])) for j in range(len(eqs))]
+
+
 def _same_affine(a, b) -> bool:
     """GroupAffine PartialEq on (xy, inf) pairs: both identity, or the same (x, y)"""
     if int(a[1]) or int(b[1]):
@@ -334,41 +348,54 @@ class ASForHadamardProducts:
         product-polynomial commitments and a*, b*; the randomness (App. C.5) is host arithmetic and the new instance (C.6) one
         3-equation msm_oneshot_batch.  -> (new instance (C1*, C2*, C3*), new witness (a*, b*, rand* | None),
         proof (hiding_comms | None, low, high))"""
-        from . import scalar_field
-        ctx, f = ck.bases.ctx, scalar_field(ck.curve)
-        m, L, n = _MODULI[f], ck.num_generators, len(witnesses)
+        ctx, L = ck.bases.ctx, ck.num_generators
         a = [np.ascontiguousarray(w[0], dtype=np.uint64).reshape(-1, 4)[:L] for w in witnesses]
         b = [np.ascontiguousarray(w[1], dtype=np.uint64).reshape(-1, 4)[:L] for w in witnesses]
         ha, hb, hr = (None, None, None) if zk is None else zk
         sess, hc = ctx.hp_prove_begin(ck.bases, a, b, L, ha, hb, hiding_index=ck.num_generators, hiding_rand=None if hr is None else np.array(hr))
+        hiding_comms = None if hc is None else [(hc[0][j], int(hc[1][j])) for j in range(3)]
+        new_instance, rand, proof, (a_star, b_star) = ASForHadamardProducts.run_session(
+            ck, sess, hiding_comms, [w[2] for w in witnesses], instances, mu_fn, nu_fn, hr, lambda nu, _: ctx.hp_prove_finish(sess, nu, L))
+        return new_instance, (a_star, b_star, rand), proof
+
+    @staticmethod
+    def run_session(ck: CommitterKey, sess: int, hiding_comms, rands, instances, mu_fn: Callable, nu_fn: Callable, hiding_rand, finish):
+        """The steps of an hp-prove session after its begin, shared by ASForHadamardProducts.prove and ASForR1CSNark.prove: mu
+        from the hiding commitments, product_poly_comm, nu, the new instance (C.6, combined_commitments), then finish(nu, new
+        instance), the caller's last call on the session, and r* (App. C.5) on the host.  rands: the pairs' (r1, r2, r3) | None;
+        hiding_rand: (hr1, hr2, hr3) with zk, else None.  The session is aborted if a step before finish fails.
+        -> (new instance, rand* | None, proof (hiding_comms | None, low, high), what finish returned)"""
+        from . import scalar_field
+        ctx, f = ck.bases.ctx, scalar_field(ck.curve)
+        m, n = _MODULI[f], len(instances)
+        zk = hiding_comms is not None
         try:
-            hiding_comms = None if hc is None else [(hc[0][j], int(hc[1][j])) for j in range(3)]
             mus = [_fe_to_int(f, x) for x in np.asarray(mu_fn(hiding_comms), dtype=np.uint64).reshape(-1, 4)]
-            mu = [1] + mus + ([mus[0] * mus[-1] % m] if zk is not None else [])
+            mu = [1] + mus + ([mus[0] * mus[-1] % m] if zk else [])
             (lo, linf), (hi, hinf) = ctx.hp_prove_product_poly_comm(sess, n, _canon_mont(f, mu))
             low = [(lo[j], int(linf[j])) for j in range(n - 1)]
             high = [(hi[j], int(hinf[j])) for j in range(n - 1)]
             nu = np.ascontiguousarray(nu_fn(low, high), dtype=np.uint64).reshape(4)
+            v = _fe_to_int(f, nu)
+            new_instance = ASForHadamardProducts.combined_commitments(ck, instances, hiding_comms, low, high, mu, v)
+            finished = finish(nu, new_instance)
         except Exception:
             try:
-                ctx.hp_prove_abort(sess)
+                ctx.hp_prove_abort(sess)       # fails harmlessly when finish itself has released the session
             except Exception:
                 pass
             raise
-        a_star, b_star = ctx.hp_prove_finish(sess, nu, L)
-        v = _fe_to_int(f, nu)
         nus = [pow(v, j, m) for j in range(2 * n - 1)]
         rand = None
-        if zk is not None:
-            hrs = [_fe_to_int(f, x) for x in hr]
-            rs = [None if w[2] is None else [_fe_to_int(f, x) for x in w[2]] for w in witnesses]
+        if zk:
+            hrs = [_fe_to_int(f, x) for x in hiding_rand]
+            rs = [None if r is None else [_fe_to_int(f, x) for x in r] for r in rands]
             mu_n = mu[n]
             r1 = (mu_n * hrs[0] + sum(mu[i] * nus[i] * rs[i][0] for i in range(n) if rs[i] is not None)) % m
             r2 = (mu[1] * hrs[1] + sum(nus[j] * rs[n - 1 - j][1] for j in range(n) if rs[n - 1 - j] is not None)) % m
             r3 = (mu_n * hrs[2] + sum(mu[i] * rs[i][2] for i in range(n) if rs[i] is not None)) * nus[n - 1] % m
             rand = [_int_to_fe(f, r) for r in (r1, r2, r3)]
-        new_instance = ASForHadamardProducts.combined_commitments(ck, instances, hiding_comms, low, high, mu, v)
-        return new_instance, (a_star, b_star, rand), (hiding_comms, low, high)
+        return new_instance, rand, (hiding_comms, low, high), finished
 
     @staticmethod
     def combined_commitments(ck: CommitterKey, instances, hiding_comms, low, high, mu, nu: int):    # :409-479 (App. C.6)
@@ -387,14 +414,7 @@ class ASForHadamardProducts:
             e1.append((hiding_comms[0], mu[n]))
             e2.append((hiding_comms[1], mu[1]))
             e3.append((hiding_comms[2], mu[n] * nus[n - 1]))
-        eqs = [e1, e2, e3]
-        width = max(len(e) for e in eqs)
-        eqs = [e + [((e[0][0][0], 1), 0)] * (width - len(e)) for e in eqs]     # (a point flagged as the identity, 0)
-        pts = np.array([[np.asarray(p[0], dtype=np.uint64) for p, _ in e] for e in eqs])
-        infs = np.array([[int(p[1]) for p, _ in e] for e in eqs], dtype=np.uint8)
-        sc = np.stack([_canon([s % m for _, s in e]) for e in eqs])
-        xy, inf = ck.bases.ctx.msm_oneshot_batch(ck.curve, pts, sc, montgomery=False, infinity=infs)
-        return tuple((xy[j], int(inf[j])) for j in range(3))
+        return tuple(_oneshot_equations(ck, [e1, e2, e3]))
 
     @staticmethod
     def verify(ck: CommitterKey, instances, new_instance, proof, mu_fn: Callable, nu_fn: Callable) -> bool:   # :815-892
@@ -514,7 +534,74 @@ class AccumulatorWitness:
 
 
 class ASForR1CSNark:
-    """The decider of src/r1cs_nark_as/mod.rs (:1031-1112) over an R1CSNark index (matrices registered once)."""
+    """The prover (:713-926) and the decider (:1031-1112) of src/r1cs_nark_as/mod.rs over an R1CSNark index (matrices
+    registered once)."""
+
+    @staticmethod
+    def prove(nark: R1CSNark, inputs, old_accumulators, gamma_fn: Callable, mu_fn: Callable, nu_fn: Callable, beta_fn: Callable, zk=None):
+        """ASForR1CSNark::prove (SURVEY App. C.12).  inputs: fresh [(r1cs_input, NarkProof)]; old_accumulators:
+        [(AccumulatorInstance, AccumulatorWitness)]; with zk there must be at least two of them together (the hp rule; the
+        caller pads).  zk = (r_x, r_w, (sigma_rA, sigma_rB, sigma_rC), ha, hb, (hr1, hr2, hr3)) from the caller's rng (ha, hb of
+        n_rows elements).  The sponge is the callables: gamma_fn(first_msg) -> gamma of a zk NARK proof, mu_fn / nu_fn as in
+        ASForHadamardProducts.prove, beta_fn(hp new instance, randomness comms | None) -> beta_1 .. beta_{n-1} (beta_n too with zk),
+        n = n_fresh + n_acc, Montgomery limbs.  One device session (accmsm_nark_as_prove_begin, product_poly_comm, finish) forms
+        the mat-vecs, the randomness and hp hiding commitments, the hp proof, a*, b* and w*; the blinded commitments of all fresh
+        inputs are ONE msm_oneshot_batch (4 equations per zk input), comm_A*, comm_B*, comm_C* another (3 equations), and x*,
+        sigma* and r* are host arithmetic.  -> (AccumulatorInstance, AccumulatorWitness, proof (hp proof, randomness comms | None))"""
+        from . import scalar_field
+        ck = nark.ck
+        ctx, f = ck.bases.ctx, scalar_field(ck.curve)
+        m, L = _MODULI[f], nark.n_rows
+        arr = lambda v: np.ascontiguousarray(v, dtype=np.uint64).reshape(-1, 4)
+        # step 2: blinded commitments (comm_M + gamma comm_rM, comm_C + gamma comm_1 + gamma^2 comm_2)
+        eqs = []
+        for _, p in inputs:
+            if p.sigmas is not None:
+                fm, g = p.first_msg, _fe_to_int(f, gamma_fn(p.first_msg))
+                eqs += [[(fm[j], 1), (fm[3 + j], g), ((fm[j][0], 1), 0)] for j in range(3)] + [[(fm[2], 1), (fm[6], g), (fm[7], g * g % m)]]
+        comb = _oneshot_equations(ck, eqs) if eqs else []
+        blinded, k = [], 0
+        for _, p in inputs:
+            fm = p.first_msg
+            if p.sigmas is None:
+                blinded.append([fm[0], fm[1], fm[2], fm[2]])
+            else:
+                blinded.append(comb[4 * k:4 * k + 4]); k += 1
+        # step 3: hp inputs, fresh first
+        hp_insts = [(b[0], b[1], b[3]) for b in blinded] + [tuple(acc.hp_instance) for acc, _ in old_accumulators]
+        hp_rands = [None if p.sigmas is None else [p.sigmas[0], p.sigmas[1], p.sigmas[3]] for _, p in inputs]
+        hp_rands += [w.hp_witness[2] for _, w in old_accumulators]
+        n, n_w = len(hp_insts), (arr(inputs[0][1].blinded_witness) if inputs else arr(old_accumulators[0][1].r1cs_blinded_witness)).shape[0]
+        r_x, r_w, sig_r, ha, hb, hr = (None,) * 6 if zk is None else zk
+        sess, hc = ctx.nark_as_prove_begin(ck.bases, nark.csr, [arr(x) for x, _ in inputs], [arr(p.blinded_witness) for _, p in inputs],
+                                           [arr(w.r1cs_blinded_witness) for _, w in old_accumulators],
+                                           [arr(w.hp_witness[0]) for _, w in old_accumulators], [arr(w.hp_witness[1]) for _, w in old_accumulators],
+                                           zk=None if zk is None else (r_x, r_w, ha, hb, np.concatenate([arr(sig_r), arr(hr)])),
+                                           hiding_index=ck.num_generators,
+                                           n_input=arr(inputs[0][0] if inputs else old_accumulators[0][0].r1cs_input).shape[0])
+        pts = None if hc is None else [(hc[0][j], int(hc[1][j])) for j in range(6)]
+        comm_r = None if pts is None else pts[3:]
+
+        def finish(nu, hp_inst):       # step 5: beta after the hp proof; step 7: w* on the device
+            beta = [1] + [_fe_to_int(f, x) for x in np.asarray(beta_fn(hp_inst, comm_r), dtype=np.uint64).reshape(-1, 4)]
+            return (beta,) + ctx.nark_as_prove_finish(sess, nu, _canon_mont(f, beta), L, n_w)
+
+        hp_inst, hp_rand, hp_proof, (beta, a_star, b_star, w_star) = ASForHadamardProducts.run_session(
+            ck, sess, None if pts is None else pts[:3], hp_rands, hp_insts, mu_fn, nu_fn, hr, finish)
+        # step 6: x*, comm_M*; step 7: sigma*, over fresh inputs, then accumulators, then (zk) the randomness
+        xs = [arr(x) for x, _ in inputs] + [arr(a.r1cs_input) for a, _ in old_accumulators] + ([arr(r_x)] if zk is not None else [])
+        x_star = np.array([_int_to_fe(f, sum(beta[k] * _fe_to_int(f, xs[k][c]) for k in range(len(xs))))
+                           for c in range(xs[0].shape[0])], dtype=np.uint64).reshape(-1, 4)
+        comms = [b[:3] for b in blinded] + [[a.comm_a, a.comm_b, a.comm_c] for a, _ in old_accumulators] + ([comm_r] if zk is not None else [])
+        comm_star = _oneshot_equations(ck, [[(c[j], beta[k]) for k, c in enumerate(comms)] for j in range(3)])
+        sigs = [None if p.sigmas is None else list(p.sigmas[:3]) for _, p in inputs] + [w.randomness for _, w in old_accumulators]
+        sigs += [list(arr(sig_r))] if zk is not None else []
+        sigma_star = None
+        if any(s is not None for s in sigs):
+            sigma_star = [_int_to_fe(f, sum(beta[k] * _fe_to_int(f, s[j]) for k, s in enumerate(sigs) if s is not None)) for j in range(3)]
+        instance = AccumulatorInstance(x_star, comm_star[0], comm_star[1], comm_star[2], tuple(hp_inst))
+        witness = AccumulatorWitness(w_star, (a_star, b_star, hp_rand), sigma_star)
+        return instance, witness, (hp_proof, comm_r)
 
     @staticmethod
     def decide(nark: R1CSNark, instance: AccumulatorInstance, witness: AccumulatorWitness) -> bool:

@@ -404,6 +404,40 @@ int accmsm_hp_prove_finish(accmsm_ctx *ctx, uint64_t session, const uint64_t nu_
                            size_t capacity, size_t *out_len);
 int accmsm_hp_prove_abort(accmsm_ctx *ctx, uint64_t session);
 
+/* ---- ASForR1CSNark::prove as a session (src/r1cs_nark_as/mod.rs:713-926; SURVEY.md App. C.12) --------------------------------
+ * An hp-prove session (above) whose first n_fresh pairs are formed on the device: the host keeps the sponge, gamma, mu, nu, beta,
+ * the blinded commitments, x*, comm_M*, sigma*, r* and C1*..C3*:
+ *     nark_as_prove_begin(fresh inputs, accumulators, zk) -> H1, H2, H3, comm_rA, comm_rB, comm_rC;  mu = sponge(..)
+ *     accmsm_hp_prove_product_poly_comm(mu) -> low, high;                                              nu, beta = sponge(..)
+ *     nark_as_prove_finish(nu, beta) -> a*, b*, w*
+ * begin: fresh input i < n_fresh is x_i (inputs[i], n_input x 4) and its NARK proof's blinded witness w'_i (n_witness x 4);
+ *   accumulator j < n_acc is its w* (acc_witnesses[j], n_witness x 4) and its hp witness a*_j, b*_j (acc_a_lens[j] /
+ *   acc_b_lens[j] <= n_rows elements).  One vector launch walks every row of A and B once for all fresh inputs and writes
+ *   A (x_i || w'_i), B (x_i || w'_i) into the session's pair buffers: the hp pairs are the fresh ones, then the accumulators'.
+ *   Zero knowledge (all of r_input (n_input x 4), r_witness (n_witness x 4), hiding_a, hiding_b (n_rows x 4 each) and
+ *   rand_mont (sigma_rA, sigma_rB, sigma_rC, r1, r2, r3: 6 x 4), or none of them): the same launch also forms M (r_x || r_w) for
+ *   M = A, B, C, k_hp_hiding_rows forms the hp hiding rows, and ONE 6-job pass over n_rows + 1 pairs returns, in this order,
+ *   Commit(ha, r1), Commit(hb, r2), Commit(ha o b_0 + a_{n-1} o hb, r3), Commit(A r, sigma_rA), Commit(B r, sigma_rB),
+ *   Commit(C r, sigma_rC) (comm_xy 6 x 8, comm_inf 6).  Without zk begin launches only the row kernel (none when n_fresh = 0).
+ *   The pass needs 6 x windows x (n_rows + 1) < 2^31: n_rows <= 27,531,840 (~2^24.7) at c = 20.
+ * product_poly_comm: accmsm_hp_prove_product_poly_comm on the same session, n = n_fresh + n_acc.
+ * finish: a* and b* as accmsm_hp_prove_finish, and w* = sum_k beta_k w_k over w'_i, then w*_j, then (zk) r_w, into w_star;
+ *   beta (beta_0 = 1 included) has n_fresh + n_acc entries, one more with zk.  finish releases the session, on error too; abort
+ *   is accmsm_hp_prove_abort.  The placeholder padding of hp (src/hp_as/mod.rs:676-710) stays with the caller.
+ * ACCMSM_E_ARG: the csr handle does not hold exactly 3 matrices; n_fresh + n_acc outside 1..16; zk with n_fresh + n_acc = 1 (the
+ * caller pads); an accumulator pair longer than n_rows, n_rows or hiding_index beyond the key, a column beyond input ||
+ * witness; a wrong n_beta; finish before product_poly_comm; accmsm_hp_prove_finish on a NARK-AS session or
+ * accmsm_nark_as_prove_finish on a plain hp session (both release it).  An unknown session: ACCMSM_E_HANDLE.  On a device group
+ * every child runs the row kernel over its rows of the key and the matrices, and child 0 forms w*; results are bit-identical. */
+int accmsm_nark_as_prove_begin(accmsm_ctx *ctx, uint64_t key_handle, uint64_t csr_handle, int n_fresh, const uint64_t *const *inputs,
+                               size_t n_input, const uint64_t *const *blinded_witnesses, size_t n_witness, int n_acc,
+                               const uint64_t *const *acc_witnesses, const uint64_t *const *acc_a, const size_t *acc_a_lens,
+                               const uint64_t *const *acc_b, const size_t *acc_b_lens, const uint64_t *r_input, const uint64_t *r_witness,
+                               const uint64_t *hiding_a, const uint64_t *hiding_b, size_t hiding_index, const uint64_t *rand_mont,
+                               uint64_t *comm_xy, uint8_t *comm_inf, uint64_t *session);
+int accmsm_nark_as_prove_finish(accmsm_ctx *ctx, uint64_t session, const uint64_t nu_mont[4], const uint64_t *beta_mont, size_t n_beta,
+                                uint64_t *a_star, uint64_t *b_star, size_t capacity, size_t *out_len, uint64_t *w_star);
+
 #ifdef __cplusplus
 }
 #endif
