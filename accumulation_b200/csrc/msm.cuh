@@ -1142,7 +1142,8 @@ __global__ void __launch_bounds__(128) k_precompute(const affine_t *__restrict__
 // replica warps on the four sub-partitions of an SM) per 32 bases runs every doubling in 3 product phases, the inversion
 // is the binary-GCD one (divergent, but nothing else competes for the SM), and the back-substitution of the windows is
 // dealt round-robin to the four replicas (every replica walks the running inverse, each converts its own windows).
-// Used by the folded keys an IpaPC::open session materialises (ipa_api.inc) and for registered keys up to 2^14 points.
+// Used by the folded keys an IpaPC::open session materialises (ipa_api.inc) and for registered keys up to 2^12 points
+// (PRECOMPUTE_COOP_MAX, accmsm.cu).
 template <int CURVE>
 __global__ void __launch_bounds__(128) k_precompute_coop(const affine_t *__restrict__ bases, uint32_t n, uint32_t c,
                                                           uint32_t nwin, affine_t *__restrict__ table) {
